@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py - clips/s of the NISQA predict hot path (BASELINE.json metric) on N B200s.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference|reference-gpu]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference|reference-gpu] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (BASELINE.json configs[1]): predict_dir bs=64, synthetic 10 s 48 kHz PCM16 clips,
@@ -17,7 +17,10 @@ engine stream), `cpu_baseline` = the oracle port on the host cores on a bounded 
 clip-parallel on all host cores) and prints the same line with "impl": "reference".
 `--impl reference-gpu` (and the `reference_gpu` key of the default line at N=1) times the UNMODIFIED
 reference torch modules in PyTorch eager on this GPU (tools/reference_gpu.py; SURVEY.md 8d's "honest thing to
-beat"), when the reference package was installed under baseline/_ref by __graft_entry__.build().
+beat"), when the reference package was installed under baseline/_ref by `tools/reference_gpu.py --install SRC`.
+`--dump-outputs DIR` (default impl): after the timed steps, rank 0 writes what the last timed step returned to its
+caller as DIR/<name>.npy (float32 scores, n_segments and status as float64; with N > 1 also the gathered rows).
+The inputs depend only on the arguments, so two builds can be compared output for output.
 """
 import argparse
 import json
@@ -450,9 +453,11 @@ def run_ours(a, rank, world, local):
         eng.set_gather_target(glob.data_ptr(), BS)
         gather = True
 
+    last_dev = {}                                # the latest step: (index, n_segments, status)
+
     def step_dev(i, sync=False):
-        eng.predict_pcm_device(dev_batches[i % N_ROT].data_ptr(), offs, n_s, srs, E.FMT_S16,
-                               scores_ring[i % 3].data_ptr(), sync=sync)
+        last_dev["out"] = (i,) + eng.predict_pcm_device(dev_batches[i % N_ROT].data_ptr(), offs, n_s, srs, E.FMT_S16,
+                                                        scores_ring[i % 3].data_ptr(), sync=sync)
 
     # e2e: the public streaming API - submit batch i (pinned host PCM16 -> H2D -> kernels -> D2H of the
     # scores), then collect batch i-1; two batches in flight, every step's copies inside the timed region
@@ -526,6 +531,13 @@ def run_ours(a, rank, world, local):
     mark0 = sampler.mark()
     ms_dev, _ = timed(step_dev, a.steps)
     launches = eng.kernel_launches() - l0
+    dump = None
+    if a.dump_outputs and rank == 0:
+        i_last, nseg_last, status_last = last_dev["out"]
+        dump = {"scores": scores_ring[i_last % 3].cpu().numpy(),
+                "n_segments": nseg_last.astype(np.float64), "status": status_last.astype(np.float64)}
+        if world > 1:
+            dump["scores_all_ranks"] = glob.cpu().numpy()
     for i in range(max(a.warmup, 4)):
         step_e2e(i)
     drain_e2e()
@@ -595,6 +607,10 @@ def run_ours(a, rank, world, local):
             "achieved_tflops_whole_step": FLOP_PER_CLIP * BS / (ms_dev / a.steps / 1e3) / 1e12,
             "parity_max_abs_vs_oracle": parity,
             "cpu_baseline": cpu_base, "reference_gpu": ref_gpu, "sharded_predict_csv": sharded}
+    if dump is not None:
+        os.makedirs(a.dump_outputs, exist_ok=True)
+        for name, arr in dump.items():
+            np.save(os.path.join(a.dump_outputs, name + ".npy"), arr)
     print(json.dumps(line), flush=True)
 
 
@@ -609,9 +625,15 @@ def main():
     ap.add_argument("--warmup-seconds", dest="warmup_seconds", type=float, default=1.5,
                     help="minimum duration of the untimed warm-up (in addition to --warmup steps)")
     ap.add_argument("--skip-cpu", dest="skip_cpu", action="store_true", help="omit the cpu_baseline leg (profiling runs)")
+    ap.add_argument("--dump-outputs", dest="dump_outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy (--impl ours)")
     a = ap.parse_args()
     if a.steps is None:
         a.steps = 200 if a.impl == "ours" else 20
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     a.warmup = max(a.warmup, 3) if a.impl == "ours" else max(a.warmup, 0)
     rank, world, local = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1)), int(os.environ.get("LOCAL_RANK", 0))
     if a.impl == "reference":

@@ -7,11 +7,10 @@ this GPU" row, the honest thing the hand-written engine has to beat.
 What runs is the UNMODIFIED reference package (``nisqa/NISQA_model.py`` + ``nisqa/NISQA_lib.py``) through its own
 public API ``nisqaModel(args).predict()`` -> ``NL.predict_dim(model, ds, bs, dev, num_workers)`` (reference
 lib:1441-1467) with the device it picks itself (CUDA when available, model:1036-1045).  The package is not part of
-this repository: ``__graft_entry__.build()`` installs a copy of ``/root/reference/nisqa`` under ``baseline/_ref/``
-(git-ignored, travels to the GPU box with the snapshot) when ``/root/reference`` exists; without it this module
-reports ``{"unavailable": ...}``.  ``librosa`` is not installable offline, so the reference's
-``lb.load / melspectrogram / amplitude_to_db`` calls land in ``oracle/librosa_compat.py`` (NumPy restatement of
-librosa 0.8.1) - stated in the output.  Nothing of the product (engine, kernels, native wav reader) is on this path.
+this repository: ``python tools/reference_gpu.py --install SRC`` copies ``SRC/nisqa`` of a NISQA checkout under
+``baseline/_ref/`` (git-ignored); without it this module reports ``{"unavailable": ...}``.  ``librosa`` is not
+installable offline, so the reference's ``lb.load / melspectrogram / amplitude_to_db`` calls land in
+``oracle/librosa_compat.py`` (NumPy restatement of librosa 0.8.1) - stated in the output.  Nothing of the product (engine, kernels, native wav reader) is on this path.
 
 Two figures:
   * ``predict_dir``: wall time of ``nisqaModel.predict()`` over a directory of synthetic 10 s 48 kHz wavs, bs=64,
@@ -37,9 +36,9 @@ if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
 
-def install_reference(src="/root/reference"):
-    """Copy of the reference package for the GPU box (pure Python, no build metadata: `pip install --target`
-    has nothing to build, the package directory IS the install).  No-op without the source tree."""
+def install_reference(src):
+    """Copy of the reference package from the NISQA checkout `src` (pure Python, no build metadata: `pip install
+    --target` has nothing to build, the package directory IS the install).  No-op without the source tree."""
     pkg = os.path.join(src, "nisqa")
     if not os.path.isdir(pkg):
         return False
@@ -111,7 +110,7 @@ def measure(n_clips=64, bs=64, seconds=10.0, sr=48000, workers=None, ckpt=None, 
     """-> dict (see module docstring).  ``ours``: optional callable(list of wav paths) -> [n, 5] scores of the
     engine on the same files, for the |delta| column."""
     if not available():
-        return {"unavailable": "baseline/_ref/nisqa is absent (installed by __graft_entry__.build() where /root/reference exists)"}
+        return {"unavailable": "baseline/_ref/nisqa is absent (install it with tools/reference_gpu.py --install SRC)"}
     import torch
     cuda = torch.cuda.is_available()
     if not cuda and not allow_cpu:           # allow_cpu: plumbing test of this module in the build container
@@ -216,10 +215,11 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--clips", type=int, default=64)
     ap.add_argument("--workers", type=int, default=None)
-    ap.add_argument("--install", action="store_true", help="copy /root/reference/nisqa to baseline/_ref and exit")
+    ap.add_argument("--install", metavar="SRC", default=None,
+                    help="copy SRC/nisqa of a NISQA checkout to baseline/_ref and exit")
     a = ap.parse_args()
     if a.install:
-        print(json.dumps({"installed": install_reference()}))
+        print(json.dumps({"installed": install_reference(a.install)}))
         return
     print(json.dumps(measure(n_clips=a.clips, workers=a.workers)))
 
