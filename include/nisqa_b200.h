@@ -264,23 +264,12 @@ NISQA_API int     nisqa_join(nisqa_engine* e);
  * with CUDA events on the engine stream when profiling was enabled; <0 if unknown.
  * groups: "frontend", "cnn", "td", "pool" */
 NISQA_API int    nisqa_set_profiling(nisqa_engine* e, int on);
-/* kernel-variant switches for A/B measurements and the parity tests:
- *   "conv_tc"    bit mask of the conv layers (2..6) that run as tcgen05 implicit GEMMs with the fp16
- *                two-term split (default / 1 = all of them); a cleared bit selects the fp32 FFMA kernel.
- *   "conv_split" 1 (default): with all of conv2..6 on tcgen05, activations travel between the layers as
- *                fp16 hi/lo plane pairs (csrc/conv_split.cu); 0: fp32 channels-last activations and the
- *                register-staged kernels of csrc/conv_tc.cu.  Results are bit-identical.
- *   "conv12"     1 (default): conv1 + pool1 + conv2 + pool2 run as ONE persistent kernel (csrc/conv12.cu), the pool1
- *                activations never reach HBM (NISQA_STAGE_POOL1 is then not dumpable); 0: separate kernels.
- *   "conv_pipe"  bit mask of the conv layers (2..6) whose plane kernel runs as persistent warp-specialised CTAs
- *                (default / 1 = all); a cleared bit selects the one-tile-per-CTA kernel.  Bit-identical results.
- *   "fe_ppc"     frame pairs per front-end CTA (0 = kernel default).
- *   "td_tiled"   1 (default): time-dependency block + pooling logits as register-tiled GEMM kernels
- *                (csrc/td_tiled.cu); 0: the one-thread-per-row kernels of csrc/td.cu.
- *   "lstm_batched" 1 (default): BiLSTM advances up to four clips per CTA in lock step; 0: one CTA per
- *                (clip, direction).
+/* options (any other name is rejected with NISQA_ERR_INVALID, "unknown option"):
+ *   "keep_pool1"  1 = also write the pool1 activations so that NISQA_STAGE_POOL1 can be dumped (default 0: the fused
+ *                 conv1 + conv2 kernel, csrc/conv12.cu, keeps them in shared memory).  Scores are unchanged.
  *   "keep_td_out" standard architecture: 1 = also store the per-step BiLSTM outputs so that
- *                NISQA_STAGE_TD_OUT can be dumped (default 0: only the final states are needed, lib:1107-1115). */
+ *                 NISQA_STAGE_TD_OUT can be dumped (default 0: only the final states are needed, lib:1107-1115).
+ *   "fe_ppc"      frame pairs per front-end CTA (0 = kernel default). */
 NISQA_API int    nisqa_set_option(nisqa_engine* e, const char* name, int value);
 NISQA_API double nisqa_group_ms(const nisqa_engine* e, const char* group);
 

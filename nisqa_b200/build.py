@@ -12,7 +12,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libnisqa_b200.so")
 STAMP = os.path.join(HERE, ".libnisqa_b200.stamp")
-SOURCES = ["engine.cu", "frontend.cu", "cnn.cu", "conv_tc.cu", "conv_split.cu", "conv12.cu", "td.cu", "td_tiled.cu", "wavio.cpp", "flac.cpp", "resample.cpp", "resample_gpu.cu"]
+SOURCES = ["engine.cu", "frontend.cu", "conv1.cu", "conv_split.cu", "conv12.cu", "td.cu", "td_tiled.cu", "wavio.cpp", "flac.cpp", "resample.cpp", "resample_gpu.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-std=c++17", "-lineinfo",
               "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden", "--shared"]
 

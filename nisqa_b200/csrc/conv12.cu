@@ -1,9 +1,8 @@
-// conv12.cu - conv1 + pool1 + conv2 + pool2 of the framewise CNN in ONE persistent kernel (round 2).
+// conv12.cu - conv1 + pool1 + conv2 + pool2 of the framewise CNN in ONE persistent kernel.
 //
-// Before: conv1_pool1_kernel (FFMA, cnn.cu) wrote the pool1 activations of every segment to HBM as fp16 plane pairs
-// (123 MB per 64-clip step) and conv_split_kernel<Conv2> read them back (202 MB) - 21 % of the CNN's DRAM traffic and
-// two launches whose CTAs spent most of their life filling / draining.  Here the pool1 tile of a segment never leaves
-// the SM: producer warps compute conv1 + BN + ReLU + pool1 of segment i+1 straight into the shared-memory image of
+// Writing pool1 to HBM as fp16 plane pairs and reading it back for conv2 would cost 123 + 202 MB per 64-clip step
+// (21 % of the CNN's DRAM traffic) and two launches whose CTAs spend most of their life filling / draining.  Here the
+// pool1 tile of a segment never leaves the SM: producer warps compute conv1 + BN + ReLU + pool1 of segment i+1 straight into the shared-memory image of
 // conv2's implicit-GEMM A operand (the plane layout of conv_split.cuh: padded rows of 16 halves, 32-byte swizzle,
 // hi / lo split) while the tensor pipe runs conv2 of segment i and the epilogue warps pool / split / store segment
 // i-1.  Reference: nisqa/NISQA_lib.py:688-695 (AdaptCNN) / 811-818 (StandardCNN).
@@ -20,8 +19,8 @@
 //   warps 17,18   MMA issuers, one per M-tile (two issuers reach the tensor pipe's rate, one does not)
 //
 // One tile = one segment (its padded 25 x 8 / 25 x 9 map is 200 / 225 of the 256 GEMM rows).  Three A buffers, two
-// accumulator sets, two staging tiles.  Arithmetic identical to conv1_pool1_kernel + conv_split_kernel<Conv2>: the
-// same fp32 conv1, the same split, the same MMAs in the same order per accumulator - bit-identical results.
+// accumulator sets, two staging tiles.  conv2 uses the two-term fp16 split of conv_split.cu and the same MMA order per
+// accumulator as conv_pipe_kernel; conv1 is conv1_cell, which conv1_pool1_kernel (conv1.cu) shares to dump pool1.
 #include <algorithm>
 #include <type_traits>
 

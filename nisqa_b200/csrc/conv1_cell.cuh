@@ -1,5 +1,6 @@
 // conv1_cell.cuh - conv1(1->16) + BN + ReLU fused with the first max-pool for ONE pooled cell of one segment (all 16
-// channels), shared by conv1_pool1_kernel (cnn.cu) and the fused conv1 + conv2 kernel (conv12.cu).
+// channels), shared by the fused conv1 + conv2 kernel (conv12.cu) and conv1_pool1_kernel (conv1.cu), which writes pool1
+// for the stage dump.
 //   MODE 0 (adapt, reference lib:690-691): adaptive_max_pool2d 48x15 -> 24x7 : rows {2i,2i+1}, cols [2j,2j+3)
 //   MODE 1 (standard, lib:813-814): MaxPool2d(2, stride 2, padding (0,1)) -> 24x8 : cols {2j-1,2j}
 #pragma once

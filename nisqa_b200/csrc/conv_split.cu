@@ -1,9 +1,25 @@
-// conv_split.cu - conv2..conv6 of the AdaptCNN / StandardCNN (reference nisqa/NISQA_lib.py:692-706,
-// 816-830) on the 5th-generation tensor cores, with the activations travelling BETWEEN the layers
-// already in the form the tensor core consumes: two fp16 planes (hi, lo) of the error-compensated
-// split  x = x_hi + x_lo  (see conv_tc.cu for the arithmetic: a_hi*[b_hi|b_lo] + a_lo*b_hi in fp32,
-// results within fp32 rounding noise of the reference), laid out in HBM as the exact shared-memory
-// image of the implicit-GEMM A tile:
+// conv_split.cu - conv3..conv6 of the AdaptCNN / StandardCNN (reference nisqa/NISQA_lib.py:696-706,
+// 820-830) as implicit GEMMs on the 5th-generation tensor cores (tcgen05 + TMEM), with the activations
+// travelling BETWEEN the layers already in the form the tensor core consumes.
+//
+// Arithmetic: an error-compensated two-term FP16 split, so that the result stays within fp32 rounding
+// noise of the reference (plain TF32 / BF16 operands move MOS by 2e-3 / 1.7e-2, SURVEY.md 0.8):
+//      a = a_hi + a_lo,  b = b_hi + b_lo      (fp16 parts: 11 + 11 significant bits)
+//      a*b ~= a_hi*b_hi + a_hi*b_lo + a_lo*b_hi          (dropped a_lo*b_lo ~ 2^-22 |a b|)
+// Issued as TWO MMAs per K-step: A_hi x [B_hi | B_lo] with N = 2*C_out (accumulator columns
+// [0,C) = hi*hi, [C,2C) = hi*lo) and A_lo x B_hi with N = C_out into columns [C,2C) as well; the
+// epilogue adds the two column halves.  Every A element is thus fetched from shared memory twice per
+// tap instead of three times.  Products are exact in the tensor core and accumulate in fp32 (TMEM).
+// The weights are pre-scaled by 2^S on the host (S chosen per layer so that max|w| 2^S <= 1024) to
+// keep b_lo out of the fp16 subnormal range; the epilogue multiplies by 2^-S (exact).  Compared with
+// 3xTF32 this halves shared memory, weight traffic and MMA time (kind::f16 has K = 16).
+//
+// GEMM view:  D[pos, co] = sum_{tap, ci} X[pos + off(tap), ci] * W[tap][co][ci]
+//   M = flattened padded positions of G segments, N = C_out, K = 9 * C_in.  The 9 taps are the SAME
+//   activation tile addressed through row-shifted descriptors, so im2col is never materialised.
+//
+// The activations are two fp16 planes (hi, lo) laid out in HBM as the exact shared-memory image of the
+// implicit-GEMM A tile:
 //
 //   plane row g(seg, hh, ww) = kSplitLead + seg * BLK + hh * P + ww,   P = W + 1, BLK = (H + 1) * P
 //     hh = 0 / ww = 0 are the shared zero row / zero column (never written: the planes are zeroed
@@ -14,11 +30,7 @@
 // so that a CTA's whole activation tile (256 + 2 * HALO consecutive rows, two planes) arrives with
 // TWO cp.async.bulk copies issued by one thread (placed at row offset g0 & 7 inside a 1024-byte
 // aligned tile so that the absolute-address swizzle of the UMMA descriptors matches the image), and
-// the producing layer's epilogue does the split once, right where the fp32 value exists.  Compared
-// with conv_tc.cu (fp32 channels-last activations, register staging + split in every consumer) the
-// fill phase of a CTA drops from ~9 k cycles of LDG -> split -> STS to one asynchronous copy, the 9
-// taps are the same tile addressed through row-shifted descriptors as before, and max-pooling runs
-// on every thread of the CTA, and 8 epilogue warps (one per TMEM lane quarter and M-tile) drain the accumulators.
+// the producing layer's epilogue does the split once, right where the fp32 value exists.
 #include <cuda_fp16.h>
 
 #include <algorithm>
@@ -27,269 +39,30 @@
 #include "tc_ptx.cuh"
 #include "conv_split.cuh"
 
-#ifndef NISQA_SP_INTERLEAVE
-#define NISQA_SP_INTERLEAVE 1      // MMA issue order: alternate the two M-tile accumulators (0: tile after tile)
-#endif
-
 namespace nisqa {
 
-#ifdef NISQA_TC_TIMING
-__device__ long long g_sp_timing[8 * 8192];
-#endif
-__device__ __forceinline__ void sp_stamp(int slot, int who, int flags) {
-#ifdef NISQA_TC_TIMING
-  if ((flags & 2) && (int)threadIdx.x == who && blockIdx.x < 8192) g_sp_timing[blockIdx.x * 8 + slot] = clock64();
-#endif
-}
-
-
-template <class C>
-__global__ void __launch_bounds__(C::NT, C::MINB)
-conv_split_kernel(const unsigned char* __restrict__ in_hi, const unsigned char* __restrict__ in_lo,
-                  const __half* __restrict__ wtc /*[9][CIN/8][hi co | lo co][8] fp16, scaled by 2^S*/,
-                  const float* __restrict__ bias, float out_scale /*2^-S*/,
-                  unsigned char* __restrict__ out_hi, unsigned char* __restrict__ out_lo,
-                  float* __restrict__ out_f32 /*last layer only*/, int n_seg, int flags) {
-  constexpr int H = C::H, W = C::W, CIN = C::CIN, COUT = C::COUT, P = C::P, BLK = C::BLK, G = C::G;
-  constexpr int HALO = C::HALO, NS = C::NSTAGE, ROWB = C::ROWB, EPW = C::EPW, MMA_TID = C::EPW * 32;
-  extern __shared__ __align__(128) unsigned char smem_raw[];
-  unsigned char* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);   // swizzle atoms repeat every 1024 B
-  const uint32_t sbase = smem_u32(smem);
-  const uint32_t a_hi = sbase + C::OFF_A_HI, a_lo = sbase + C::OFF_A_LO, b_base = sbase + C::OFF_B;
-  const uint32_t bar_full = sbase + C::OFF_BAR;          // [NS]
-  const uint32_t bar_empty = bar_full + 8 * NS;          // [NS]
-  const uint32_t bar_acc = bar_full + 16 * NS;
-  const uint32_t bar_a = bar_acc + 8;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(smem + C::OFF_BAR + 16 * NS + 16);
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const int seg0 = blockIdx.x * G;
-  const int g0 = kSplitLead + seg0 * BLK - HALO;         // first plane row of this CTA's tile
-  const uint32_t sh = (uint32_t)(g0 & 7);                // tile row == plane row (mod 8)
-  sp_stamp(0, 0, flags);
-
-  if (warp == 0) tmem_alloc(smem_u32(tmem_slot), C::TMEM_COLS);
-  if (tid == 32) {
-#pragma unroll
-    for (int i = 0; i < NS; ++i) { mbar_init(bar_full + 8 * i, 1); mbar_init(bar_empty + 8 * i, 1); }
-    mbar_init(bar_acc, 1);
-    mbar_init(bar_a, 1);
-    fence_barrier_init();
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem = *tmem_slot;
-  sp_stamp(1, 0, flags);
-
-  if (warp == EPW + 1) {
-    // ===== producer (one lane): the activation tile (2 copies), then the weights tap by tap =====
-    if (lane == 0) {
-      constexpr uint32_t A_COPY = (uint32_t)C::AROWS * ROWB;
-      mbar_expect_tx(bar_a, 2 * A_COPY);
-      bulk_g2s(a_hi + sh * ROWB, in_hi + (size_t)g0 * ROWB, A_COPY, bar_a);
-      bulk_g2s(a_lo + sh * ROWB, in_lo + (size_t)g0 * ROWB, A_COPY, bar_a);
-      for (int t = 0; t < 9; ++t) {
-        const int s = t % NS;
-        if (t >= NS) mbar_wait(bar_empty + 8 * s, ((t / NS) - 1) & 1);     // MMAs of tap t-NS have drained the stage
-        mbar_expect_tx(bar_full + 8 * s, C::B_STAGE);
-        bulk_g2s(b_base + s * C::B_STAGE, wtc + (size_t)t * (C::B_STAGE / 2), C::B_STAGE, bar_full + 8 * s);
-      }
-    }
-  } else if (warp == EPW) {
-    // ===== MMA issuer (one lane) =====
-    if (lane == 0) {
-      mbar_wait(bar_a, 0);
-      sp_stamp(2, MMA_TID, flags);
-      for (int t = 0; t < 9; ++t) {
-        const int s = t % NS;
-        mbar_wait(bar_full + 8 * s, (t / NS) & 1);
-        if (t == 0) sp_stamp(6, MMA_TID, flags);
-        tc_fence_after();
-        const int tapoff = (t / 3 - 1) * P + (t % 3 - 1);
-        const uint32_t bst = b_base + s * C::B_STAGE;       // [ci/8][2*COUT rows: hi then lo][8 halves]
-#if NISQA_SP_INTERLEAVE
-        // Consecutive MMAs alternate between the two M-tiles: an MMA that accumulates into the tile the
-        // previous one wrote waits for it (the tensor pipe was 39 % busy = exactly the useful math while the
-        // MMA phases covered more than half of the time), so the two independent accumulators are interleaved
-        // (hi 0, hi 1, lo 0, lo 1 per K-step).  Per accumulator the order of additions is unchanged.
-        const uint32_t row0 = sh + (uint32_t)(HALO + tapoff);
-#pragma unroll
-        for (int ks = 0; ks < CIN / 16; ++ks) {
-          const uint64_t db = make_desc(bst + (uint32_t)(2 * ks) * (2 * COUT * 16), 2 * COUT * 16, 128);
-          const uint32_t aoff0 = row0 * ROWB + (uint32_t)ks * 32, aoff1 = aoff0 + 128u * ROWB;
-          umma_f16(tmem, make_desc_swz(a_hi + aoff0, 8 * ROWB, C::LAYOUT), db, C::IDESC_2N, (t | ks) != 0);   // tile 0: [0,C) += hi*hi ; [C,2C) += hi*lo
-          umma_f16(tmem + 2 * COUT, make_desc_swz(a_hi + aoff1, 8 * ROWB, C::LAYOUT), db, C::IDESC_2N, (t | ks) != 0);   // tile 1
-          // lo*hi joins hi*lo in the SMALL accumulator [C,2C): the tensor core truncates every accumulation at the
-          // accumulator's own magnitude, so the main accumulator only ever sees the 9 * C_in / 16 hi*hi terms
-          umma_f16(tmem + COUT, make_desc_swz(a_lo + aoff0, 8 * ROWB, C::LAYOUT), db, C::IDESC_1N, 1);            // tile 0: [C,2C) += lo*hi
-          umma_f16(tmem + 3 * COUT, make_desc_swz(a_lo + aoff1, 8 * ROWB, C::LAYOUT), db, C::IDESC_1N, 1);        // tile 1
-        }
-#else   // A/B: one M-tile after the other (every MMA depends on its predecessor)
-#pragma unroll
-        for (int mt = 0; mt < 2; ++mt) {
-          const uint32_t row = sh + (uint32_t)(HALO + mt * 128 + tapoff);
-          const uint32_t d = tmem + mt * (2 * COUT);
-#pragma unroll
-          for (int ks = 0; ks < CIN / 16; ++ks) {
-            const uint32_t aoff = row * ROWB + (uint32_t)ks * 32;
-            const uint64_t db = make_desc(bst + (uint32_t)(2 * ks) * (2 * COUT * 16), 2 * COUT * 16, 128);
-            umma_f16(d, make_desc_swz(a_hi + aoff, 8 * ROWB, C::LAYOUT), db, C::IDESC_2N, (t | ks) != 0);
-            umma_f16(d + COUT, make_desc_swz(a_lo + aoff, 8 * ROWB, C::LAYOUT), db, C::IDESC_1N, 1);
-          }
-        }
-#endif
-        umma_commit(bar_empty + 8 * s);          // stage s may be refilled once these MMAs retire
-      }
-      umma_commit(bar_acc);                      // all accumulators final
-      sp_stamp(7, MMA_TID, flags);
-    }
-  } else {
-    // ===== epilogue part 1: warp w reads TMEM lanes 32 (w & 3) .. +31 (its M-tile(s)) =====
-    mbar_wait(bar_acc, 0);
-    tc_fence_after();
-    sp_stamp(3, 0, flags);
-    float* stg = reinterpret_cast<float*>(smem);          // reuses the A/B region (all MMAs retired)
-    const int quarter = warp & 3;
-    const int mt_begin = (EPW == 8) ? (warp >> 2) : 0, mt_end = (EPW == 8) ? (warp >> 2) + 1 : 2;
-#pragma unroll 1
-    for (int mt = mt_begin; mt < mt_end; ++mt) {
-      const int r = mt * 128 + quarter * 32 + lane;
-      const int s = r / BLK, q = r - s * BLK;
-      const int hh = q / P, ww = q - hh * P;
-      const bool live = (s < G) && (seg0 + s < n_seg);          // this TMEM row maps to a plane row that is stored
-      bool valid = live && hh >= 1 && ww >= 1;                  // ... and to an interior position
-      if (C::CENTER) valid = valid && (ww == 2);
-      const uint32_t trow = tmem + ((uint32_t)(quarter * 32) << 16) + mt * (2 * COUT);
-#pragma unroll 1
-      for (int c16 = 0; c16 < COUT / 16; ++c16) {          // 16 output channels per step
-        uint32_t ra[16], rb[16];
-        tmem_ld16_nowait(trow + c16 * 16, ra);             // hi*hi
-        tmem_ld16_nowait(trow + COUT + c16 * 16, rb);      // hi*lo + lo*hi
-        tmem_ld_wait();
-        float v[16];
-        const float4* b4 = reinterpret_cast<const float4*>(bias + c16 * 16);
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          const float4 bb = __ldg(b4 + j);
-          v[4 * j + 0] = fmaxf(fmaf(__uint_as_float(ra[4 * j + 0]) + __uint_as_float(rb[4 * j + 0]), out_scale, bb.x), 0.f);
-          v[4 * j + 1] = fmaxf(fmaf(__uint_as_float(ra[4 * j + 1]) + __uint_as_float(rb[4 * j + 1]), out_scale, bb.y), 0.f);
-          v[4 * j + 2] = fmaxf(fmaf(__uint_as_float(ra[4 * j + 2]) + __uint_as_float(rb[4 * j + 2]), out_scale, bb.z), 0.f);
-          v[4 * j + 3] = fmaxf(fmaf(__uint_as_float(ra[4 * j + 3]) + __uint_as_float(rb[4 * j + 3]), out_scale, bb.w), 0.f);
-        }
-        if constexpr (C::POOL != SP_POOL_NONE) {
-          if (valid) {
-            float4* dst = reinterpret_cast<float4*>(stg + ((s * H + (hh - 1)) * W + (ww - 1)) * C::STG_STRIDE + c16 * 16);
-#pragma unroll
-            for (int j = 0; j < 4; ++j) dst[j] = make_float4(v[4 * j], v[4 * j + 1], v[4 * j + 2], v[4 * j + 3]);
-          }
-        } else if constexpr (C::OUT_SPLIT) {
-          // image row r <-> plane row g = g_out0 + r (same padded geometry as the input); the zero row /
-          // column positions are written as zeros, so the whole image goes out as one contiguous block
-          if (live) {
-            const int g = kSplitLead + seg0 * BLK + r;
-            const size_t img0 = (size_t)(kSplitLead + seg0 * BLK) * C::OROWB;
-#pragma unroll
-            for (int j = 0; j < 2; ++j) {
-              uint4 hi = make_uint4(0u, 0u, 0u, 0u), lo = hi;
-              if (valid)
-                split8(make_float4(v[8 * j], v[8 * j + 1], v[8 * j + 2], v[8 * j + 3]),
-                       make_float4(v[8 * j + 4], v[8 * j + 5], v[8 * j + 6], v[8 * j + 7]), hi, lo);
-              const uint32_t o = (uint32_t)(split_off<C::OROWB>(g, c16 * 2 + j) - img0);
-              *reinterpret_cast<uint4*>(smem + o) = hi;
-              *reinterpret_cast<uint4*>(smem + C::IMG_BYTES + o) = lo;
-            }
-          }
-        } else {
-          if (valid) {
-            const int w = C::CENTER ? 0 : ww - 1;
-            float4* dst = reinterpret_cast<float4*>(stg + ((s * H + (hh - 1)) * C::WO + w) * COUT + c16 * 16);
-#pragma unroll
-            for (int j = 0; j < 4; ++j) dst[j] = make_float4(v[4 * j], v[4 * j + 1], v[4 * j + 2], v[4 * j + 3]);
-          }
-        }
-      }
-    }
-    if constexpr (C::POOL == SP_POOL_NONE) fence_proxy_async();     // staged image -> visible to the bulk store
-  }
-  sp_stamp(4, 0, flags);
-  tc_fence_before();
-  __syncthreads();                     // accumulators read, staging tile complete; every role is done
-  if (warp == 0) tmem_dealloc(tmem, C::TMEM_COLS);
-
-  if constexpr (C::POOL == SP_POOL_NONE) {
-    // ===== epilogue part 2: one thread writes the staged image with bulk stores =====
-    if (tid == 32) {
-      const int nvalid = min(G, n_seg - seg0);
-      if constexpr (C::OUT_SPLIT) {
-        const size_t img0 = (size_t)(kSplitLead + seg0 * BLK) * C::OROWB;
-        const uint32_t bytes = (uint32_t)nvalid * C::OBLK * C::OROWB;
-        bulk_s2g(out_hi + img0, sbase, bytes);
-        bulk_s2g(out_lo + img0, sbase + C::IMG_BYTES, bytes);
-      } else {
-        const uint32_t per_seg = C::HO * C::WO * COUT * 4;
-        bulk_s2g(out_f32 + (size_t)seg0 * (per_seg / 4), sbase, (uint32_t)nvalid * per_seg);
-      }
-      bulk_commit();
-      bulk_wait_read0();               // shared memory must outlive the reads of the bulk stores
-    }
-  }
-  if constexpr (C::POOL != SP_POOL_NONE) {
-    // ===== epilogue part 2 (all threads): max-pool the staged tile, split, store =====
-    const float* stg = reinterpret_cast<const float*>(smem);
-    constexpr int POW = C::POW, HO = H / 2, C8 = COUT / 8;
-    for (int it = tid; it < G * HO * POW * C8; it += C::NT) {
-      const int c8 = it % C8;
-      int rest = it / C8;
-      const int pw = rest % POW; rest /= POW;
-      const int ph = rest % HO;
-      const int s = rest / HO;
-      if (seg0 + s >= n_seg) continue;
-      int x0, x1;
-      if (C::POOL == SP_POOL_ADAPT) { x0 = (pw * W) / POW; x1 = ((pw + 1) * W + POW - 1) / POW; }
-      else { x0 = 2 * pw; x1 = 2 * pw + 2; }
-      float4 ma = make_float4(0.f, 0.f, 0.f, 0.f), mb = ma;       // post-ReLU values are >= 0
-      for (int hy = 2 * ph; hy < 2 * ph + 2; ++hy)
-        for (int x = x0; x < x1; ++x) {
-          const float4* t = reinterpret_cast<const float4*>(stg + ((s * H + hy) * W + x) * C::STG_STRIDE + c8 * 8);
-          const float4 ta = t[0], tb = t[1];
-          ma.x = fmaxf(ma.x, ta.x); ma.y = fmaxf(ma.y, ta.y); ma.z = fmaxf(ma.z, ta.z); ma.w = fmaxf(ma.w, ta.w);
-          mb.x = fmaxf(mb.x, tb.x); mb.y = fmaxf(mb.y, tb.y); mb.z = fmaxf(mb.z, tb.z); mb.w = fmaxf(mb.w, tb.w);
-        }
-      uint4 hi, lo;
-      split8(ma, mb, hi, lo);
-      const int g = kSplitLead + (seg0 + s) * C::OBLK + (ph + 1) * C::OP + (pw + 1);
-      const size_t o = split_off<C::OROWB>(g, c8);
-      *reinterpret_cast<uint4*>(out_hi + o) = hi;
-      *reinterpret_cast<uint4*>(out_lo + o) = lo;
-    }
-  }
-  sp_stamp(5, 0, flags);
-}
-
-// =====================================================================================================
-// Persistent, warp-specialised variant (round 2).  Measured on B200 (profiles/r02b_mma_probe_issuers.txt): one
-// issuing thread retires a M=128 K=16 MMA every ~96 cycles whatever N is; two issuers (two CTAs, or two warps of
-// one CTA) overlap until the pipe's own floor binds (N=128: 64 cycles = 8 KB of operands at 128 B/clk; N=64: 48
-// cycles, operand-fetch bound).  In conv_split_kernel above the two co-resident CTAs of an SM therefore saturate the
-// tensor pipe WHILE both are in their MMA phase - and leave it idle during fill, epilogue and teardown (47 % of
+// Persistent, warp-specialised kernel.  Measured on B200 (profiles/r02b_mma_probe_issuers.txt): one issuing thread
+// retires a M=128 K=16 MMA every ~96 cycles whatever N is; two issuers (two CTAs, or two warps of one CTA) overlap
+// until the pipe's own floor binds (N=128: 64 cycles = 8 KB of operands at 128 B/clk; N=64: 48 cycles, operand-fetch
+// bound).  A CTA that runs one tile and exits leaves the tensor pipe idle during fill, epilogue and teardown (47 % of
 // the time on conv4).  Here ONE CTA per SM stays resident and walks over its tiles with every phase overlapped:
 //
 //   warps 0..7   epilogue of tile i-1 (TMEM -> registers -> staging -> pool / split -> HBM)
 //   warp  8      producer: activation tile of tile i+1 (two bulk copies) as soon as its buffer is free
-//   warp  9      producer: weights, tap by tap through a ring (or ONCE, when all nine taps fit: conv2 / conv3)
+//   warp  9      producer: weights, tap by tap through a ring (or ONCE, when all nine taps fit: conv3)
 //   warps 10,11  MMA issuers of tile i, one per M-tile (two issuers reach the pipe's rate, one does not)
 //
 // Two activation buffers and two accumulator sets (2 x 4 C_out TMEM columns) alternate; the epilogue stages its
 // tile in the activation buffer it has just finished with, so a buffer returns to the producer when the tile's
-// output has left it.  Same planes, same MMAs on the same values in the same order per accumulator as
-// conv_split_kernel: results are bit-identical (tests/test_gpu_parity.py::test_conv_paths_agree).
+// output has left it.
+//
+// -DNISQA_TC_TIMING: each layer L (3..6) accumulates per-CTA cycle counters in its own block of g_pipe_timing
+// (tools/pipe_timing.py).
 #ifdef NISQA_TC_TIMING
-__device__ long long g_pipe_timing[256 * 16];       // per CTA: cycles accumulated per role / wait (tools/pipe_timing.py)
-#define PIPE_T0() const long long _pt0 = clock64()
-#define PIPE_ACC(slot) do { if (blockIdx.x < 256) g_pipe_timing[blockIdx.x * 16 + (slot)] += clock64() - _pt0; } while (0)
+__device__ long long g_pipe_timing[4 * 256 * 16];   // [layer - 3][CTA][slot]
 #define PIPE_NOW() clock64()
-#define PIPE_ADD(slot, t0) do { if (blockIdx.x < 256) g_pipe_timing[blockIdx.x * 16 + (slot)] += clock64() - (t0); } while (0)
-#define PIPE_COUNT(slot, n) do { if (blockIdx.x < 256) g_pipe_timing[blockIdx.x * 16 + (slot)] += (n); } while (0)
+#define PIPE_ADD(slot, t0) do { if (blockIdx.x < 256) g_pipe_timing[((L - 3) * 256 + blockIdx.x) * 16 + (slot)] += clock64() - (t0); } while (0)
+#define PIPE_COUNT(slot, n) do { if (blockIdx.x < 256) g_pipe_timing[((L - 3) * 256 + blockIdx.x) * 16 + (slot)] += (n); } while (0)
 #else
 #define PIPE_NOW() 0ll
 #define PIPE_ADD(slot, t0) do { (void)(t0); } while (0)
@@ -303,28 +76,12 @@ struct PipeCfg {
                                                              : (C::OUT_SPLIT ? 2 : 1) * C::IMG_BYTES;
   static constexpr int BUF_RAW = (2 * C::A_BYTES > STG_BYTES) ? 2 * C::A_BYTES : STG_BYTES;
   static constexpr int BUF_BYTES = (BUF_RAW + 1023) & ~1023;
-#ifndef NISQA_PIPE_SEP
-#define NISQA_PIPE_SEP 0      // measured: 0 (shared buffers) 0.164 ms, 1 0.187 ms, 2 0.177 ms for conv3 (profiles/r02z_ab_kernels.txt)
-#endif
-  // EXPERIMENT (off): un-pooled layers whose output image is larger than the activation tile (conv3) with two dedicated
-  // activation buffers and separate staging, so that the next tile's activations are fetched as soon as the MMAs of tile
-  // it-2 have retired, not after its epilogue has staged and shipped its output (34 % of conv3's issue time waits for
-  // that).  Measured slower: with ONE staging buffer the 60 KB image's way out of the SM (~3 600 cycles) serialises with
-  // the next tile's staging; with two, the weights no longer fit and stream through the ring.
-  static constexpr int A_PAIR = (2 * C::A_BYTES + 1023) & ~1023;
-  static constexpr int STG_AL = (STG_BYTES + 1023) & ~1023;
-  // NISQA_PIPE_SEP: 1 = one staging buffer, weights resident; 2 = two staging buffers, weights through a 4-stage ring
-  static constexpr int NSTG = NISQA_PIPE_SEP == 2 ? 2 : 1;
-  static constexpr bool SEP_STAGE = NISQA_PIPE_SEP && C::POOL == SP_POOL_NONE && STG_BYTES > 2 * C::A_BYTES &&
-                                    2 * A_PAIR + NSTG * STG_AL + (NSTG == 2 ? 4 : 9) * C::B_STAGE <= 227 * 1024 - 2048;
-  static constexpr int A_STRIDE = SEP_STAGE ? A_PAIR : BUF_BYTES;       // bytes between the two activation buffers
-  static constexpr int OFF_STG = 2 * A_PAIR;                            // (SEP_STAGE) the staging buffer(s)
-  static constexpr int AB_BYTES = SEP_STAGE ? 2 * A_PAIR + NSTG * STG_AL : 2 * BUF_BYTES;
-  static constexpr bool RESIDENT = (SEP_STAGE && NSTG == 1) || (!SEP_STAGE && AB_BYTES + 9 * C::B_STAGE <= 196 * 1024);      // all nine taps stay in shared memory
+  static constexpr int AB_BYTES = 2 * BUF_BYTES;                       // two activation buffers (also the staging tiles)
+  static constexpr bool RESIDENT = AB_BYTES + 9 * C::B_STAGE <= 196 * 1024;     // all nine taps stay in shared memory
   static constexpr int NSW = RESIDENT ? 9 : ((AB_BYTES + 4 * C::B_STAGE <= 216 * 1024) ? 4 : 3);
   static constexpr int OFF_B = AB_BYTES;
   static constexpr int OFF_BAR = OFF_B + NSW * C::B_STAGE;
-  static constexpr int N_BAR = 2 + 2 + 2 * NSW + 2 + 2 + 2 + 2;
+  static constexpr int N_BAR = 2 + 2 + 2 * NSW + 2 + 2 + 2;
   static constexpr int SMEM_BYTES = OFF_BAR + 8 * N_BAR + 32 + 1024;
   static constexpr int COLS_TILE = 4 * C::COUT;                        // 2 M-tiles x [hi*hi+lo*hi | hi*lo]
   static constexpr int TMEM_ALLOC = 2 * COLS_TILE;                     // 512 (C_out 64) / 256 (C_out 32): powers of two
@@ -332,7 +89,7 @@ struct PipeCfg {
   static_assert(TMEM_ALLOC == 256 || TMEM_ALLOC == 512, "TMEM allocation");
 };
 
-template <class C>
+template <class C, int L>
 __global__ void __launch_bounds__(PipeCfg<C>::NT, 1)
 conv_pipe_kernel(const unsigned char* __restrict__ in_hi, const unsigned char* __restrict__ in_lo,
                  const __half* __restrict__ wtc, const float* __restrict__ bias, float out_scale,
@@ -349,21 +106,18 @@ conv_pipe_kernel(const unsigned char* __restrict__ in_hi, const unsigned char* _
   const uint32_t bar0 = sbase + Pc::OFF_BAR;
   const uint32_t bar_a_full = bar0, bar_a_free = bar0 + 16, bar_b_full = bar0 + 32, bar_b_empty = bar_b_full + 8 * NSW;
   const uint32_t bar_acc_full = bar_b_empty + 8 * NSW, bar_acc_free = bar_acc_full + 16, bar_stage_ready = bar_acc_free + 16;
-  const uint32_t bar_stg_free = bar_stage_ready + 16;              // (SEP_STAGE) the shipped image has left the staging buffer
-  constexpr bool SEP = Pc::SEP_STAGE;
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(smem + Pc::OFF_BAR + 8 * Pc::N_BAR + 8);
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
 
   if (warp == 0) tmem_alloc(smem_u32(tmem_slot), Pc::TMEM_ALLOC);
   if (tid == 256) {
     for (int i = 0; i < 2; ++i) {
-      mbar_init(bar_a_full + 8 * i, 1); mbar_init(bar_a_free + 8 * i, SEP ? 2 : 1);   // SEP: both MMA issuers commit
+      mbar_init(bar_a_full + 8 * i, 1); mbar_init(bar_a_free + 8 * i, 1);
       mbar_init(bar_acc_full + 8 * i, 2);          // both MMA issuers commit
       mbar_init(bar_acc_free + 8 * i, 8);          // one arrival per epilogue warp
       mbar_init(bar_stage_ready + 8 * i, 8);       // un-pooled layers: the staged output image is complete
     }
     for (int i = 0; i < NSW; ++i) { mbar_init(bar_b_full + 8 * i, 1); mbar_init(bar_b_empty + 8 * i, 2); }
-    mbar_init(bar_stg_free, 1); mbar_init(bar_stg_free + 8, 1);
     fence_barrier_init();
   }
   tc_fence_before();
@@ -379,11 +133,10 @@ conv_pipe_kernel(const unsigned char* __restrict__ in_hi, const unsigned char* _
       constexpr uint32_t A_COPY = (uint32_t)C::AROWS * ROWB;
       auto store_tile = [&](int j) {
         const int b = j & 1;
-        if constexpr (SEP && Pc::NSTG == 1) mbar_wait(bar_stage_ready, j & 1);      // one staging buffer: a completion per tile
-        else mbar_wait(bar_stage_ready + 8 * b, (j >> 1) & 1);     // all eight epilogue warps have staged tile j
+        mbar_wait(bar_stage_ready + 8 * b, (j >> 1) & 1);          // all eight epilogue warps have staged tile j
         const int seg0 = (blockIdx.x + j * (int)gridDim.x) * G;
         const int nvalid = min(G, n_seg - seg0);
-        const uint32_t sb = SEP ? sbase + Pc::OFF_STG + (Pc::NSTG == 2 ? b * Pc::STG_AL : 0) : sbase + b * Pc::BUF_BYTES;
+        const uint32_t sb = sbase + b * Pc::BUF_BYTES;
         if constexpr (C::OUT_SPLIT) {
           const size_t img0 = (size_t)(kSplitLead + seg0 * BLK) * C::OROWB;
           const uint32_t bytes = (uint32_t)nvalid * C::OBLK * C::OROWB;
@@ -395,23 +148,20 @@ conv_pipe_kernel(const unsigned char* __restrict__ in_hi, const unsigned char* _
         }
         bulk_commit();
         bulk_wait_read0();                                         // the stores have read the buffer
-        if constexpr (SEP) mbar_arrive(bar_stg_free + (Pc::NSTG == 2 ? 8 * b : 0));
       };
       int it = 0;
       for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x, ++it) {
         const int buf = it & 1, ph = (it >> 1) & 1;
         const long long tw = PIPE_NOW();
-        if constexpr (SEP) mbar_wait(bar_a_free + 8 * buf, ph ^ 1);           // the MMAs of tile it-2 have read the buffer
-        else if constexpr (C::POOL == SP_POOL_NONE) { if (it >= 2) store_tile(it - 2); }
+        if constexpr (C::POOL == SP_POOL_NONE) { if (it >= 2) store_tile(it - 2); }
         else mbar_wait(bar_a_free + 8 * buf, ph ^ 1);              // the pooling epilogue of tile it-2 has left the buffer
         PIPE_ADD(9, tw);
         const int g0 = kSplitLead + tile * G * BLK - HALO;
         const uint32_t sh = (uint32_t)(g0 & 7);
-        const uint32_t a_hi = sbase + buf * Pc::A_STRIDE, a_lo = a_hi + C::A_BYTES;
+        const uint32_t a_hi = sbase + buf * Pc::BUF_BYTES, a_lo = a_hi + C::A_BYTES;
         mbar_expect_tx(bar_a_full + 8 * buf, 2 * A_COPY);
         bulk_g2s(a_hi + sh * ROWB, in_hi + (size_t)g0 * ROWB, A_COPY, bar_a_full + 8 * buf);
         bulk_g2s(a_lo + sh * ROWB, in_lo + (size_t)g0 * ROWB, A_COPY, bar_a_full + 8 * buf);
-        if constexpr (SEP) { if (it >= 2) store_tile(it - 2); }    // (its epilogue started when those MMAs retired)
       }
       if constexpr (C::POOL == SP_POOL_NONE)
         for (int j = (it >= 2 ? it - 2 : 0); j < it; ++j) store_tile(j);
@@ -449,7 +199,7 @@ conv_pipe_kernel(const unsigned char* __restrict__ in_hi, const unsigned char* _
         tc_fence_after();
         const int g0 = kSplitLead + tile * G * BLK - HALO;
         const uint32_t sh = (uint32_t)(g0 & 7);
-        const uint32_t a_hi = sbase + buf * Pc::A_STRIDE, a_lo = a_hi + C::A_BYTES;
+        const uint32_t a_hi = sbase + buf * Pc::BUF_BYTES, a_lo = a_hi + C::A_BYTES;
         const uint32_t d = tmem + buf * Pc::COLS_TILE + mt * (2 * COUT);
         for (int t = 0; t < 9; ++t, ++cnt) {
           const int s = Pc::RESIDENT ? t : cnt % NSW;
@@ -471,7 +221,6 @@ conv_pipe_kernel(const unsigned char* __restrict__ in_hi, const unsigned char* _
           }
           if (!Pc::RESIDENT) umma_commit(bar_b_empty + 8 * s);
         }
-        if constexpr (SEP) umma_commit(bar_a_free + 8 * buf);      // the activation buffer may be refilled
         umma_commit(bar_acc_full + 8 * buf);
       }
       if (mt == 0) { PIPE_ADD(4, t_all); PIPE_COUNT(15, it); }
@@ -483,15 +232,11 @@ conv_pipe_kernel(const unsigned char* __restrict__ in_hi, const unsigned char* _
     for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x, ++it) {
       const int buf = it & 1, ph = (it >> 1) & 1;
       const int seg0 = tile * G;
-      unsigned char* sbuf = SEP ? smem + Pc::OFF_STG + (Pc::NSTG == 2 ? buf * Pc::STG_AL : 0) : smem + buf * Pc::BUF_BYTES;   // staging = the tile's own activation buffer, or the one staging buffer
+      unsigned char* sbuf = smem + buf * Pc::BUF_BYTES;          // staging = the tile's own activation buffer
       float* stg = reinterpret_cast<float*>(sbuf);
       long long tw = PIPE_NOW();
       mbar_wait(bar_acc_full + 8 * buf, ph);                     // every MMA of the tile has retired
       if (tid == 0) PIPE_ADD(5, tw);
-      if constexpr (SEP) {                                       // the image of tile it-1 (it-2) has left the staging buffer
-        if constexpr (Pc::NSTG == 1) mbar_wait(bar_stg_free, (it & 1) ^ 1);
-        else mbar_wait(bar_stg_free + 8 * buf, ph ^ 1);
-      }
       tw = PIPE_NOW();
       tc_fence_after();
       {
@@ -555,7 +300,7 @@ conv_pipe_kernel(const unsigned char* __restrict__ in_hi, const unsigned char* _
       if constexpr (C::POOL == SP_POOL_NONE) {
         fence_proxy_async();                                       // staged image -> visible to the producer's bulk stores
         __syncwarp();
-        if (lane == 0) mbar_arrive((SEP && Pc::NSTG == 1) ? bar_stage_ready : bar_stage_ready + 8 * buf);
+        if (lane == 0) mbar_arrive(bar_stage_ready + 8 * buf);
         if (tid == 0) PIPE_ADD(6, tw);
       } else {
         if (tid == 0) PIPE_ADD(6, tw);
@@ -627,7 +372,7 @@ __global__ void unsplit_kernel(const unsigned char* __restrict__ hi, const unsig
 }
 
 
-template <class C>
+template <class C, int L>
 static void launch_pipe(cudaStream_t st, const unsigned char* in_hi, const unsigned char* in_lo, const __half* wtc,
                         const float* b, float scale, unsigned char* out_hi, unsigned char* out_lo, float* out_f32,
                         int n_seg) {
@@ -635,27 +380,14 @@ static void launch_pipe(cudaStream_t st, const unsigned char* in_hi, const unsig
   static unsigned long long configured = 0;
   static int n_sm = 0;
   if (first_launch_on_device(configured)) {
-    cudaFuncSetAttribute(conv_pipe_kernel<C>, cudaFuncAttributeMaxDynamicSharedMemorySize, Pc::SMEM_BYTES);
+    cudaFuncSetAttribute(conv_pipe_kernel<C, L>, cudaFuncAttributeMaxDynamicSharedMemorySize, Pc::SMEM_BYTES);
     int dev = 0;
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev);
   }
   const int n_tiles = (n_seg + C::G - 1) / C::G;
   const int grid = std::min(n_tiles, n_sm > 0 ? n_sm : 148);
-  conv_pipe_kernel<C><<<grid, Pc::NT, Pc::SMEM_BYTES, st>>>(in_hi, in_lo, wtc, b, scale, out_hi, out_lo, out_f32, n_seg, n_tiles);
-}
-
-template <class C>
-static void launch_sp(cudaStream_t st, const unsigned char* in_hi, const unsigned char* in_lo, const __half* wtc,
-                      const float* b, float scale, unsigned char* out_hi, unsigned char* out_lo, float* out_f32,
-                      int n_seg, int flags) {
-  if (flags & 4) { launch_pipe<C>(st, in_hi, in_lo, wtc, b, scale, out_hi, out_lo, out_f32, n_seg); return; }
-  static unsigned long long configured = 0;
-  if (first_launch_on_device(configured)) {
-    cudaFuncSetAttribute(conv_split_kernel<C>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM_BYTES);
-  }
-  conv_split_kernel<C><<<(n_seg + C::G - 1) / C::G, C::NT, C::SMEM_BYTES, st>>>(
-      in_hi, in_lo, wtc, b, scale, out_hi, out_lo, out_f32, n_seg, flags);
+  conv_pipe_kernel<C, L><<<grid, Pc::NT, Pc::SMEM_BYTES, st>>>(in_hi, in_lo, wtc, b, scale, out_hi, out_lo, out_f32, n_seg, n_tiles);
 }
 
 // Geometry of the plane pair that feeds conv layer `layer` (2..6): rows of the padded image per segment,
@@ -672,11 +404,11 @@ size_t split_plane_bytes(int std_mode, int layer, int n_seg) {
   return (rows * (size_t)C * 2 + 1023) & ~(size_t)1023;
 }
 
-// conv layer 2..6 on planes; the last layer (6) writes the fp32 CNN features (adapt: [seg][6][64];
+// conv layer 3..6 on planes; the last layer (6) writes the fp32 CNN features (adapt: [seg][6][64];
 // standard: [seg][6][2][64])
 void launch_conv_split(cudaStream_t st, int std_mode, int layer, const void* in_hi, const void* in_lo,
                        const void* wtc, const float* b, float out_scale, void* out_hi, void* out_lo,
-                       float* out_f32, int n_seg, int flags) {
+                       float* out_f32, int n_seg) {
   const __half* w = reinterpret_cast<const __half*>(wtc);
   const unsigned char* ih = static_cast<const unsigned char*>(in_hi);
   const unsigned char* il = static_cast<const unsigned char*>(in_lo);
@@ -684,19 +416,17 @@ void launch_conv_split(cudaStream_t st, int std_mode, int layer, const void* in_
   unsigned char* ol = static_cast<unsigned char*>(out_lo);
   if (!std_mode) {
     switch (layer) {
-      case 2: launch_sp<SpConv2A>(st, ih, il, w, b, out_scale, oh, ol, out_f32, n_seg, flags); break;
-      case 3: launch_sp<SpConv3A>(st, ih, il, w, b, out_scale, oh, ol, out_f32, n_seg, flags); break;
-      case 4: launch_sp<SpConv4A>(st, ih, il, w, b, out_scale, oh, ol, out_f32, n_seg, flags); break;
-      case 5: launch_sp<SpConv5A>(st, ih, il, w, b, out_scale, oh, ol, out_f32, n_seg, flags); break;
-      default: launch_sp<SpConv6A>(st, ih, il, w, b, out_scale, oh, ol, out_f32, n_seg, flags); break;
+      case 3: launch_pipe<SpConv3A, 3>(st, ih, il, w, b, out_scale, oh, ol, out_f32, n_seg); break;
+      case 4: launch_pipe<SpConv4A, 4>(st, ih, il, w, b, out_scale, oh, ol, out_f32, n_seg); break;
+      case 5: launch_pipe<SpConv5A, 5>(st, ih, il, w, b, out_scale, oh, ol, out_f32, n_seg); break;
+      default: launch_pipe<SpConv6A, 6>(st, ih, il, w, b, out_scale, oh, ol, out_f32, n_seg); break;
     }
   } else {
     switch (layer) {
-      case 2: launch_sp<SpConv2S>(st, ih, il, w, b, out_scale, oh, ol, out_f32, n_seg, flags); break;
-      case 3: launch_sp<SpConv3S>(st, ih, il, w, b, out_scale, oh, ol, out_f32, n_seg, flags); break;
-      case 4: launch_sp<SpConv4S>(st, ih, il, w, b, out_scale, oh, ol, out_f32, n_seg, flags); break;
-      case 5: launch_sp<SpConv5S>(st, ih, il, w, b, out_scale, oh, ol, out_f32, n_seg, flags); break;
-      default: launch_sp<SpConv6S>(st, ih, il, w, b, out_scale, oh, ol, out_f32, n_seg, flags); break;
+      case 3: launch_pipe<SpConv3S, 3>(st, ih, il, w, b, out_scale, oh, ol, out_f32, n_seg); break;
+      case 4: launch_pipe<SpConv4S, 4>(st, ih, il, w, b, out_scale, oh, ol, out_f32, n_seg); break;
+      case 5: launch_pipe<SpConv5S, 5>(st, ih, il, w, b, out_scale, oh, ol, out_f32, n_seg); break;
+      default: launch_pipe<SpConv6S, 6>(st, ih, il, w, b, out_scale, oh, ol, out_f32, n_seg); break;
     }
   }
 }
@@ -714,12 +444,9 @@ void launch_unsplit(cudaStream_t st, int std_mode, int layer, const void* hi, co
 }
 
 #ifdef NISQA_TC_TIMING
-int sp_timing_read(long long* host, int n) {
-  return (int)cudaMemcpyFromSymbol(host, g_sp_timing, sizeof(long long) * n);
-}
 int pipe_timing_read(long long* host, int n, int reset) {
   int rc = (int)cudaMemcpyFromSymbol(host, g_pipe_timing, sizeof(long long) * n);
-  if (reset) { static long long zero[256 * 16]; cudaMemcpyToSymbol(g_pipe_timing, zero, sizeof zero); }
+  if (reset) { static long long zero[4 * 256 * 16]; cudaMemcpyToSymbol(g_pipe_timing, zero, sizeof zero); }
   return rc;
 }
 #endif

@@ -1,6 +1,5 @@
 // conv_split.cuh - geometry / layout of the fp16 plane pairs shared by the tcgen05 conv kernels (conv_split.cu:
-// one tile per CTA and the persistent pipelined variant; conv12.cu: conv1 + conv2 fused).  See conv_split.cu for
-// the layout description.
+// conv3..conv6; conv12.cu: conv1 + conv2 fused).  See conv_split.cu for the layout description.
 #pragma once
 #include <cuda_fp16.h>
 
@@ -19,12 +18,8 @@ __device__ __forceinline__ size_t split_off(int g, int c) {
   return o ^ ((o >> 3) & (size_t)(ROWB - 16));
 }
 
-template <int H_, int W_, int CIN_, int COUT_, int POOL_, int POW_, int NSTAGE_, int EPW_, bool F32OUT_ = false, bool CENTER_ = false>
+template <int H_, int W_, int CIN_, int COUT_, int POOL_, int POW_, bool F32OUT_ = false, bool CENTER_ = false>
 struct SpCfg {
-  static constexpr int EPW = EPW_;                // epilogue warps: 4 (each owns both M-tiles of its TMEM lane quarter)
-                                                  // or 8 (warp w: lane quarter w & 3, M-tile w >> 2)
-  static constexpr int NT = (EPW + 2) * 32;       // + MMA issuer warp + producer warp
-  static_assert(EPW_ == 4 || EPW_ == 8, "epilogue warps");
   static constexpr int H = H_, W = W_, CIN = CIN_, COUT = COUT_, POOL = POOL_, POW = POW_;
   static constexpr bool CENTER = CENTER_;         // conv6 of the AdaptCNN: kernel (3,3), padding (1,0) on a
                                                   // 3-wide map == the padded conv evaluated at column 1 only
@@ -40,60 +35,36 @@ struct SpCfg {
   static constexpr int NCH = CIN / 8;             // 16-byte K chunks (8 halves)
   static constexpr int B_HALF = NCH * COUT * 16;  // per hi / lo
   static constexpr int B_STAGE = 2 * B_HALF;
-  static constexpr int NSTAGE = NSTAGE_;
-  static constexpr int TMEM_COLS = (4 * COUT <= 64) ? 64 : (4 * COUT <= 128 ? 128 : 256);   // 2 M-tiles x 2*COUT
   // output geometry (= the next layer's input geometry)
   static constexpr int HO = (POOL == SP_POOL_NONE) ? H : H / 2;
   static constexpr int WO = (POOL == SP_POOL_NONE) ? (CENTER ? 1 : W) : POW;
   static constexpr int OP = WO + 1, OBLK = (HO + 1) * OP, OROWB = COUT * 2;
   static constexpr int STG_STRIDE = COUT + 4;     // floats per staged row (conflict-free float4)
-  static constexpr int OFF_A_HI = 0;
-  static constexpr int OFF_A_LO = A_BYTES;
-  static constexpr int OFF_B = 2 * A_BYTES;
-  static constexpr int OFF_BAR = OFF_B + NSTAGE * B_STAGE;
-  static constexpr int SMEM_BYTES = OFF_BAR + 16 * NSTAGE + 32 + 1024;    // + slack: the tile is aligned to 1024 B
-  static constexpr int MINB_SMEM = (SMEM_BYTES <= 56 * 1024) ? 4 : (SMEM_BYTES <= 74 * 1024) ? 3 : (SMEM_BYTES <= 112 * 1024 ? 2 : 1);
-  static constexpr int MINB = (MINB_SMEM * TMEM_COLS <= 512) ? MINB_SMEM : 512 / TMEM_COLS;
   // D=f32, A=B=f16, both K-major, M=128; N = 2*COUT ([b_hi|b_lo]) and N = COUT (b_hi only)
   static constexpr uint32_t IDESC_2N = (1u << 4) | ((uint32_t)((2 * COUT) >> 3) << 17) | ((128u >> 4) << 24);
   static constexpr uint32_t IDESC_1N = (1u << 4) | ((uint32_t)(COUT >> 3) << 17) | ((128u >> 4) << 24);
-  static_assert(POOL == SP_POOL_NONE || G * H * W * STG_STRIDE * 4 <= 2 * A_BYTES + NSTAGE * B_STAGE,
-                "pool staging tile must fit in the A+B region");
   // un-pooled layers stage their output in shared memory as the exact HBM image of the CTA's segments
   // (plane rows incl. the zero row / column, or the fp32 feature rows) and write it with bulk stores
   static constexpr int IMG_BYTES = OUT_SPLIT ? G * OBLK * OROWB : G * HO * WO * COUT * 4;
-  static_assert(POOL != SP_POOL_NONE || (OUT_SPLIT ? 2 : 1) * IMG_BYTES <= OFF_BAR, "output image must fit in the A+B region");
   static_assert(B_STAGE % 16 == 0 && CIN % 16 == 0 && COUT % 32 == 0, "shape");
   static_assert(ROWB == 32 || ROWB == 64 || ROWB == 128, "rows are 32 / 64 / 128 bytes (one swizzle atom)");
   static_assert(HALO <= kSplitLead, "kSplitLead");
   static_assert(!CENTER || F32OUT_, "the centre-column variant only exists as the last layer");
   static_assert(OUT_SPLIT || POOL == SP_POOL_NONE, "fp32 output is not pooled");
-  static_assert(G >= 1 && MINB * TMEM_COLS <= 512, "tile / TMEM budget");
+  static_assert(G >= 1, "tile");
 };
 
-#ifndef NISQA_SP_NS4
-#define NISQA_SP_NS4 2
-#endif
-#ifndef NISQA_SP_NS5
-#define NISQA_SP_NS5 2
-#endif
-#ifndef NISQA_SP_NS3
-#define NISQA_SP_NS3 4
-#endif
-// layers 2..6; std_mode selects the StandardCNN geometry (W 8/4/2, MaxPool2d(2))
-#ifndef NISQA_SP_EPW
-#define NISQA_SP_EPW 8
-#endif
-//                     H   W  CIN COUT POOL           POW NSTAGE        EPW          F32OUT CENTER
-using SpConv2A = SpCfg<24, 7, 16, 32, SP_POOL_ADAPT, 5, 9, 4>;          // 4 CTAs / SM: registers only allow 6 warps
-using SpConv3A = SpCfg<12, 5, 32, 64, SP_POOL_NONE, 0, NISQA_SP_NS3, NISQA_SP_EPW>;
-using SpConv4A = SpCfg<12, 5, 64, 64, SP_POOL_ADAPT, 3, NISQA_SP_NS4, NISQA_SP_EPW>;
-using SpConv5A = SpCfg<6, 3, 64, 64, SP_POOL_NONE, 0, NISQA_SP_NS5, NISQA_SP_EPW>;
-using SpConv6A = SpCfg<6, 3, 64, 64, SP_POOL_NONE, 0, NISQA_SP_NS5, NISQA_SP_EPW, true, true>;
-using SpConv2S = SpCfg<24, 8, 16, 32, SP_POOL_2X2, 4, 9, 4>;
-using SpConv3S = SpCfg<12, 4, 32, 64, SP_POOL_NONE, 0, 4, NISQA_SP_EPW>;
-using SpConv4S = SpCfg<12, 4, 64, 64, SP_POOL_2X2, 2, 2, NISQA_SP_EPW>;
-using SpConv5S = SpCfg<6, 2, 64, 64, SP_POOL_NONE, 0, 2, NISQA_SP_EPW>;
-using SpConv6S = SpCfg<6, 2, 64, 64, SP_POOL_NONE, 0, 2, NISQA_SP_EPW, true>;
+// layers 2..6; std_mode selects the StandardCNN geometry (W 8/4/2, MaxPool2d(2)).  conv2 runs only inside conv12_kernel.
+//                     H   W  CIN COUT POOL           POW F32OUT CENTER
+using SpConv2A = SpCfg<24, 7, 16, 32, SP_POOL_ADAPT, 5>;
+using SpConv3A = SpCfg<12, 5, 32, 64, SP_POOL_NONE, 0>;
+using SpConv4A = SpCfg<12, 5, 64, 64, SP_POOL_ADAPT, 3>;
+using SpConv5A = SpCfg<6, 3, 64, 64, SP_POOL_NONE, 0>;
+using SpConv6A = SpCfg<6, 3, 64, 64, SP_POOL_NONE, 0, true, true>;
+using SpConv2S = SpCfg<24, 8, 16, 32, SP_POOL_2X2, 4>;
+using SpConv3S = SpCfg<12, 4, 32, 64, SP_POOL_NONE, 0>;
+using SpConv4S = SpCfg<12, 4, 64, 64, SP_POOL_2X2, 2>;
+using SpConv5S = SpCfg<6, 2, 64, 64, SP_POOL_NONE, 0>;
+using SpConv6S = SpCfg<6, 2, 64, 64, SP_POOL_NONE, 0, true>;
 
 }  // namespace nisqa

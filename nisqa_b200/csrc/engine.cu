@@ -27,24 +27,19 @@ void launch_frontend(cudaStream_t, const void*, int, const ClipDesc*, int, int,
 void launch_seg_table(cudaStream_t, const ClipDesc*, int, const int*, const unsigned*, int, int,
                       int*, float*, int*);
 void launch_mel_dump(cudaStream_t, const float*, const ClipDesc*, int, const unsigned*, float*);
-// cnn.cu
+// conv1.cu
 void launch_conv1(cudaStream_t, int, const float*, const int*, const float*, const float*,
-                  const float*, float*, int, void*, void*);
-void launch_conv_layer(cudaStream_t, int, int, const float*, const float*, const float*, float*, int);
+                  const float*, void*, void*, int);
 void launch_nhwc_to_nchw(cudaStream_t, const float*, float*, long long, int, int);
-// conv_tc.cu
-void launch_conv_tc(cudaStream_t, int, int, const float*, const void*, const float*, float, float*, int);
 // conv_split.cu
 size_t split_plane_bytes(int std_mode, int layer, int n_seg);
 void launch_conv_split(cudaStream_t, int, int, const void*, const void*, const void*, const float*, float,
-                       void*, void*, float*, int, int);
+                       void*, void*, float*, int);
 void launch_unsplit(cudaStream_t, int, int, const void*, const void*, float*, int);
 // conv12.cu
 void launch_conv12(cudaStream_t, int, const float*, const int*, const float*, const float*, const float*, const void*,
                    const float*, float, void*, void*, int);
 #ifdef NISQA_TC_TIMING
-int tc_timing_read(long long*, int);
-int sp_timing_read(long long*, int);
 int pipe_timing_read(long long*, int, int);
 int c12_timing_read(long long*, int, int);
 #endif
@@ -56,7 +51,6 @@ struct SaLayerParams {
 struct PoolHeadParams { const float* W1T; const float* b1; const float* w2; const float* b2; const float* w3; const float* b3; };
 struct LstmParams { const float* w_ih; const float* w_hh; const float* b; const float* w_pool; };
 void launch_fc20(cudaStream_t, const float*, const float*, const float*, float*, int);
-void launch_lstm(cudaStream_t, const float*, const ClipDesc*, int, const LstmParams&, float*, float*, float, float*);
 void launch_lstm_batched(cudaStream_t, const float*, const ClipDesc*, const int*, int, const LstmParams&, float*, float*, float, float*);
 void launch_pool_final(cudaStream_t, const float*, const float*, const ClipDesc*, int, const PoolHeadParams&, int, int, float*);
 // td_tiled.cu
@@ -154,13 +148,12 @@ constexpr int kLanes = NISQA_LANES;
 constexpr int kStages = 6;     // staging slots / submissions in flight (uploads run ahead of the lanes)
 struct Lane {
   cudaStream_t stream = nullptr;
-  DevBuf mel, segtab, act1, act2, act3, act4, act5, feats, xa, xb, qkv, qkv2, logits, feats20, tdout, partial, fused, td2in, ffa, ffb;
-  DevBuf planes[7];        // planes[l]: fp16 hi | lo plane pair feeding conv layer l (2..6), conv_split.cu
+  DevBuf mel, segtab, feats, xa, xb, qkv, qkv2, logits, feats20, tdout, partial, fused, td2in, ffa, ffb;
+  DevBuf planes[7];        // planes[l]: fp16 hi | lo plane pair feeding conv layer l (3..6; 2: pool1, keep_pool1 only), conv_split.cu
   size_t plane_bytes[7] = {0, 0, 0, 0, 0, 0, 0};   // offset of the lo plane inside planes[l] (half of the allocation)
   void release() {
     for (auto& b : planes) b.release();
-    DevBuf* all[] = {&mel, &segtab, &act1, &act2, &act3, &act4, &act5,
-                     &feats, &xa, &xb, &qkv, &qkv2, &logits, &feats20, &tdout, &partial, &fused, &td2in, &ffa, &ffb};
+    DevBuf* all[] = {&mel, &segtab, &feats, &xa, &xb, &qkv, &qkv2, &logits, &feats20, &tdout, &partial, &fused, &td2in, &ffa, &ffb};
     for (auto* b : all) b->release();
     if (stream) cudaStreamDestroy(stream);
   }
@@ -200,15 +193,9 @@ struct nisqa_engine {
   bool weights_loaded = false;
   bool profiling = false;
   int fe_ppc = 0;          // frame pairs per front-end CTA (0: kernel default)
-  int conv12 = 1;          // conv1 + pool1 + conv2 + pool2 in one persistent kernel (conv12.cu): pool1 never reaches HBM
-  bool last_conv12 = false;
-  int conv_pipe = 0x78;    // bit l (conv2's small tiles are faster one per CTA, four CTAs per SM): conv2..6 plane kernels as persistent warp-specialised CTAs (conv_pipe_kernel); 0: one tile per CTA
-  int conv_split = 1;      // conv2..6 exchange activations as fp16 hi/lo plane pairs (conv_split.cu); needs conv_tc == 0x7c
-  int tc_timing_layer = 0; // NISQA_TC_TIMING builds: the layer whose CTAs record their phase stamps
-  bool last_split = false; // the last pass ran the plane pipeline (stage dumps convert back to fp32)
-  int lstm_batched = 1;    // BiLSTM: NB clips per CTA in lock step (td.cu lstm_batched_kernel); 0: one CTA per (clip, direction)
+  int keep_pool1 = 0;      // also write pool1 to the plane pair planes[2] (conv12_kernel keeps it on chip; only the stage dump reads it)
+  bool last_pool1 = false; // the last pass wrote pool1
   int keep_td_out = 0;     // standard arch: also write the per-step LSTM outputs [n_seg][256] (only the stage dump reads them)
-  int conv_tc = 0x7c;      // bit l set: conv layer l (2..6) runs on tcgen05 (fp16 two-term split); else fp32 FFMA
   std::vector<TimerSlot> timers;
 
   // weights arena (device) + offsets
@@ -236,7 +223,7 @@ struct nisqa_engine {
   int64_t pass_counter = 0;
   Ticket tickets[kStages];
   int64_t next_ticket = 1;
-  DevBuf scores, dump;
+  DevBuf scores, dump, dump_nhwc;     // stage dumps: the NCHW result, and the channels-last activations it is converted from
 
   // description of the last pass (stage dumps)
   std::vector<ClipDesc> last_clips;
@@ -252,7 +239,7 @@ struct nisqa_engine {
 
   ~nisqa_engine() {
     for (auto* f : fbs) { f->window.release(); f->band_start.release(); f->band_k0.release(); f->weights.release(); f->wtab.release(); delete f; }
-    DevBuf* all[] = {&warena, &fb_table, &tw4096, &scores, &dump, &rs_raw, &rs_out, &rs_clips, &rs_times, &rs_win};
+    DevBuf* all[] = {&warena, &fb_table, &tw4096, &scores, &dump, &dump_nhwc, &rs_raw, &rs_out, &rs_clips, &rs_times, &rs_win};
     rs_host.release();
     for (auto* b : all) b->release();
     h_scores.release();
@@ -451,7 +438,8 @@ struct Packer {
   }
 };
 
-bool pack_conv(Packer& P, int idx, int cin, int cout) {
+// BatchNorm-folded conv weights go to `wf` as [cin][9][cout]; the folded bias goes to the arena as conv<idx>.b
+bool pack_conv(Packer& P, int idx, int cin, int cout, std::vector<float>& wf) {
   char nm[96];
   auto name = [&](const char* fmt) { snprintf(nm, sizeof nm, fmt, idx); return std::string(nm); };
   const TensorView* w = P.get(name("cnn.model.conv%d.weight"), {cout, cin, 3, 3});
@@ -461,7 +449,7 @@ bool pack_conv(Packer& P, int idx, int cin, int cout) {
   const TensorView* mu = P.get(name("cnn.model.bn%d.running_mean"), {cout});
   const TensorView* var = P.get(name("cnn.model.bn%d.running_var"), {cout});
   if (!w || !b || !g || !be || !mu || !var) return false;
-  const size_t wo = P.alloc(name("conv%d.w"), (size_t)cin * 9 * cout);
+  wf.assign((size_t)cin * 9 * cout, 0.f);
   const size_t bo = P.alloc(name("conv%d.b"), cout);
   for (int co = 0; co < cout; ++co) {
     // eval-mode BatchNorm2d (eps 1e-5) folded into the convolution (SURVEY.md Appendix A)
@@ -469,8 +457,7 @@ bool pack_conv(Packer& P, int idx, int cin, int cout) {
     P.arena[bo + co] = (float)(((double)b->d[co] - (double)mu->d[co]) * s + (double)be->d[co]);
     for (int ci = 0; ci < cin; ++ci)
       for (int tap = 0; tap < 9; ++tap)
-        P.arena[wo + ((size_t)ci * 9 + tap) * cout + co] =
-            (float)((double)w->d[((size_t)co * cin + ci) * 9 + tap] * s);
+        wf[((size_t)ci * 9 + tap) * cout + co] = (float)((double)w->d[((size_t)co * cin + ci) * 9 + tap] * s);
   }
   return true;
 }
@@ -538,16 +525,21 @@ int pack_weights(nisqa_engine* e, const nisqa_tensor* tensors, int n) {
     }
     if (!ok) return fail(e, NISQA_ERR_WEIGHTS, P.missing);
   }
-  for (int i = 1; conv_net && i <= 6; ++i)
-    if (!pack_conv(P, i, cin[i], cout[i])) return fail(e, NISQA_ERR_WEIGHTS, P.missing);
-  // conv2..conv6 for the tcgen05 path: [tap][ci/8][hi co | lo co][8] fp16 two-term split of w * 2^S
-  for (int i = 2; conv_net && i <= 6; ++i) {
-    char k1[32], k2[32];
-    snprintf(k1, sizeof k1, "conv%d.w", i); snprintf(k2, sizeof k2, "conv%d.wtc", i);
-    const int ci_n = cin[i], co_n = cout[i], nch = ci_n / 8;
-    const size_t src = e->woff.at(k1);
+  // conv1 runs on FFMA with the fp32 weights; conv2..conv6 on tcgen05 with [tap][ci/8][hi co | lo co][8], the fp16
+  // two-term split of w * 2^S (conv_split.cu)
+  std::vector<float> wf;
+  for (int i = 1; conv_net && i <= 6; ++i) {
+    if (!pack_conv(P, i, cin[i], cout[i], wf)) return fail(e, NISQA_ERR_WEIGHTS, P.missing);
+    if (i == 1) {
+      const size_t o = P.alloc("conv1.w", wf.size());
+      memcpy(&P.arena[o], wf.data(), wf.size() * 4);
+      continue;
+    }
+    char k2[32];
+    snprintf(k2, sizeof k2, "conv%d.wtc", i);
+    const int ci_n = cin[i], co_n = cout[i];
     float wmax = 0.f;
-    for (size_t j = 0; j < (size_t)ci_n * 9 * co_n; ++j) wmax = std::max(wmax, fabsf(P.arena[src + j]));
+    for (float w : wf) wmax = std::max(wmax, fabsf(w));
     int S = 0;
     while (S < 14 && wmax * (float)(2 << S) <= 1024.f) ++S;        // max|w| * 2^S <= 1024
     e->tc_scale[i] = 1.0f / (float)(1 << S);
@@ -556,7 +548,7 @@ int pack_weights(nisqa_engine* e, const nisqa_tensor* tensors, int n) {
     for (int tap = 0; tap < 9; ++tap)
       for (int ci = 0; ci < ci_n; ++ci)
         for (int co = 0; co < co_n; ++co) {
-          const float w = P.arena[src + ((size_t)ci * 9 + tap) * co_n + co] * (float)(1 << S);
+          const float w = wf[((size_t)ci * 9 + tap) * co_n + co] * (float)(1 << S);
           const __half hi = __float2half_rn(w);
           const __half lo = __float2half_rn(w - __half2float(hi));
           __half* base = reinterpret_cast<__half*>(&P.arena[dst]) + (size_t)tap * 2 * ci_n * co_n;
@@ -564,7 +556,6 @@ int pack_weights(nisqa_engine* e, const nisqa_tensor* tensors, int n) {
           const size_t off = ((size_t)(ci / 8) * (2 * co_n) + co) * 8 + (ci & 7);
           base[off] = hi;
           base[off + (size_t)co_n * 8] = lo;
-          (void)nch;
         }
   }
 
@@ -905,27 +896,17 @@ int run_pass(nisqa_engine* e, const PassInput& in) {
     CK(cudaEventRecord(SG.ev_copied, cs));
     CK(cudaStreamWaitEvent(st, SG.ev_copied, 0));
     // ---- workspaces
-    const int W1 = std_mode ? 8 : 7, W2 = std_mode ? 4 : 5, W3 = std_mode ? 2 : 3;
     const int FEAT = std_mode ? 768 : 384;
     CK(LN.mel.reserve((size_t)n_frames * kMels * 4));
     CK(LN.segtab.reserve((size_t)n_seg * 12));
-    const bool split = e->conv_split && e->conv_tc == 0x7c;
-    e->last_split = split;
     const bool conv_net = c.cnn_kind == NISQA_CNN_CONV;
-    if (!conv_net) {
-    } else if (split) {
-      for (int l = (e->conv12 ? 3 : 2); l <= 6; ++l) {
-        // the lo plane sits at a fixed offset of the ALLOCATION (not of this pass's n_seg): the zero rows /
-        // columns of both planes must stay where they were when the buffer was cleared
-        CK(LN.planes[l].reserve_zeroed(2 * split_plane_bytes(std_mode, l, n_seg), st));
-        LN.plane_bytes[l] = (LN.planes[l].cap / 2) & ~(size_t)1023;
-      }
-    } else {
-      CK(LN.act1.reserve((size_t)n_seg * 24 * W1 * 16 * 4));
-      CK(LN.act2.reserve((size_t)n_seg * 12 * W2 * 32 * 4));
-      CK(LN.act3.reserve((size_t)n_seg * 12 * W2 * 64 * 4));
-      CK(LN.act4.reserve((size_t)n_seg * 6 * W3 * 64 * 4));
-      CK(LN.act5.reserve((size_t)n_seg * 6 * W3 * 64 * 4));
+    const bool keep_pool1 = conv_net && e->keep_pool1;
+    e->last_pool1 = keep_pool1;
+    for (int l = keep_pool1 ? 2 : 3; conv_net && l <= 6; ++l) {
+      // the lo plane sits at a fixed offset of the ALLOCATION (not of this pass's n_seg): the zero rows /
+      // columns of both planes must stay where they were when the buffer was cleared
+      CK(LN.planes[l].reserve_zeroed(2 * split_plane_bytes(std_mode, l, n_seg), st));
+      LN.plane_bytes[l] = (LN.planes[l].cap / 2) & ~(size_t)1023;
     }
     CK(LN.feats.reserve((size_t)n_seg * FEAT * 4));
     int* seg_frame0 = LN.segtab.as<int>();
@@ -941,8 +922,6 @@ int run_pass(nisqa_engine* e, const PassInput& in) {
                        seg_frame0, seg_thr, seg_clip); }
     auto plane_hi = [&](int l) { return LN.planes[l].as<char>(); };
     auto plane_lo = [&](int l) { return LN.planes[l].as<char>() + LN.plane_bytes[l]; };
-    const bool fused12 = split && e->conv12;
-    e->last_conv12 = fused12;
     const float* sa_in = LN.feats.as<float>();       // rows fed to the first self-attention stack
     int sa_nk = 6;                                   // ... in 64-wide chunks
     if (!conv_net) {
@@ -966,35 +945,23 @@ int run_pass(nisqa_engine* e, const PassInput& in) {
           sa_in = LN.ffa.as<float>();
         }
       }
-    } else if (fused12) {
-      Scope s(e, "conv12");
-      launch_conv12(st, std_mode, LN.mel.as<float>(), seg_frame0, seg_thr, W(e, "conv1.w"), W(e, "conv1.b"),
-                    W(e, "conv2.wtc"), W(e, "conv2.b"), e->tc_scale[2], plane_hi(3), plane_lo(3), n_seg);
     } else {
-      Scope s(e, "conv1");
-      launch_conv1(st, std_mode, LN.mel.as<float>(), seg_frame0, seg_thr, W(e, "conv1.w"),
-                   W(e, "conv1.b"), split ? nullptr : LN.act1.as<float>(), n_seg,
-                   split ? plane_hi(2) : nullptr, split ? plane_lo(2) : nullptr);
-    }
-    if (conv_net) {
-      const float* cin_[7] = {nullptr, nullptr, LN.act1.as<float>(), LN.act2.as<float>(), LN.act3.as<float>(),
-                              LN.act4.as<float>(), LN.act5.as<float>()};
-      float* cout_[7] = {nullptr, nullptr, LN.act2.as<float>(), LN.act3.as<float>(), LN.act4.as<float>(),
-                         LN.act5.as<float>(), LN.feats.as<float>()};
-      for (int l = fused12 ? 3 : 2; l <= 6; ++l) {
-        char nm[16], kw[24], kt[24], kb[24];
-        snprintf(nm, sizeof nm, "conv%d", l); snprintf(kw, sizeof kw, "conv%d.w", l);
+      if (keep_pool1) {     // (not a "conv*" scope: the cnn group and the per-kernel tables count the product path only)
+        Scope s(e, "pool1_dump");
+        launch_conv1(st, std_mode, LN.mel.as<float>(), seg_frame0, seg_thr, W(e, "conv1.w"), W(e, "conv1.b"),
+                     plane_hi(2), plane_lo(2), n_seg);
+      }
+      { Scope s(e, "conv12");
+        launch_conv12(st, std_mode, LN.mel.as<float>(), seg_frame0, seg_thr, W(e, "conv1.w"), W(e, "conv1.b"),
+                      W(e, "conv2.wtc"), W(e, "conv2.b"), e->tc_scale[2], plane_hi(3), plane_lo(3), n_seg); }
+      for (int l = 3; l <= 6; ++l) {
+        char nm[16], kt[24], kb[24];
+        snprintf(nm, sizeof nm, "conv%d", l);
         snprintf(kt, sizeof kt, "conv%d.wtc", l); snprintf(kb, sizeof kb, "conv%d.b", l);
         Scope s(e, nm);
-        if (split)
-          launch_conv_split(st, std_mode, l, plane_hi(l), plane_lo(l), W(e, kt), W(e, kb), e->tc_scale[l],
-                            l < 6 ? plane_hi(l + 1) : nullptr, l < 6 ? plane_lo(l + 1) : nullptr,
-                            l == 6 ? LN.feats.as<float>() : nullptr, n_seg,
-                            (e->tc_timing_layer == l ? 2 : 0) | (((e->conv_pipe >> l) & 1) ? 4 : 0));
-        else if (e->conv_tc & (1 << l))
-          launch_conv_tc(st, std_mode, l, cin_[l], W(e, kt), W(e, kb), e->tc_scale[l], cout_[l], n_seg);
-        else
-          launch_conv_layer(st, std_mode, l, cin_[l], W(e, kw), W(e, kb), cout_[l], n_seg);
+        launch_conv_split(st, std_mode, l, plane_hi(l), plane_lo(l), W(e, kt), W(e, kb), e->tc_scale[l],
+                          l < 6 ? plane_hi(l + 1) : nullptr, l < 6 ? plane_lo(l + 1) : nullptr,
+                          l == 6 ? LN.feats.as<float>() : nullptr, n_seg);
       }
     }
 
@@ -1101,19 +1068,15 @@ int run_pass(nisqa_engine* e, const PassInput& in) {
       const bool lastbi = c.pool == NISQA_POOL_LAST_STEP_BI;
       const bool keep = e->keep_td_out || !lastbi;        // the other pooling modules read every step's output
       { Scope s(e, "lstm", 2);
-        if (e->lstm_batched)
-          launch_lstm_batched(st, LN.feats20.as<float>(), d_clips, d_by_len, n, L, keep ? LN.tdout.as<float>() : nullptr,
-                              LN.partial.as<float>(), e->pool_bias_std, lastbi ? scores : nullptr);
-        else
-          launch_lstm(st, LN.feats20.as<float>(), d_clips, n, L, LN.tdout.as<float>(), LN.partial.as<float>(), e->pool_bias_std,
-                      lastbi ? scores : nullptr); }
+        launch_lstm_batched(st, LN.feats20.as<float>(), d_clips, d_by_len, n, L, keep ? LN.tdout.as<float>() : nullptr,
+                            LN.partial.as<float>(), e->pool_bias_std, lastbi ? scores : nullptr); }
       if (!lastbi) {
         Scope s(e, "pool");
         PoolSimpleParams Q = {W(e, "pool.a1"), W(e, "pool.a1b"), W(e, "pool.w3"), W(e, "pool.b3")};
         launch_pool_simple(st, LN.tdout.as<float>(), 256, d_clips, n, c.pool, Q, 1, max_n_seg, scores);
       }
       e->last_td_in = nullptr;
-      e->last_td_out = (e->lstm_batched && !keep) ? nullptr : LN.tdout.as<float>();
+      e->last_td_out = keep ? LN.tdout.as<float>() : nullptr;
     }
   }
   CK(cudaGetLastError());
@@ -1484,13 +1447,14 @@ int64_t nisqa_stage_dump(nisqa_engine* e, int stage, float* out, int64_t cap) {
   int64_t count = 0;
   const float* src = nullptr;
   int hw = 0, ch = 0;    // NHWC -> NCHW conversion when ch > 0
+  int plane_layer = 0;   // the stage lives in the plane pair feeding this conv layer
   switch (stage) {
     case NISQA_STAGE_MEL_DB: count = (int64_t)e->last_n_frames * kMels; break;
-    case NISQA_STAGE_POOL1: src = LN.act1.as<float>(); hw = 24 * W1; ch = 16; break;
-    case NISQA_STAGE_POOL2: src = LN.act2.as<float>(); hw = 12 * W2; ch = 32; break;
-    case NISQA_STAGE_CONV3: src = LN.act3.as<float>(); hw = 12 * W2; ch = 64; break;
-    case NISQA_STAGE_POOL3: src = LN.act4.as<float>(); hw = 6 * W3; ch = 64; break;
-    case NISQA_STAGE_CONV5: src = LN.act5.as<float>(); hw = 6 * W3; ch = 64; break;
+    case NISQA_STAGE_POOL1: plane_layer = 2; hw = 24 * W1; ch = 16; break;
+    case NISQA_STAGE_POOL2: plane_layer = 3; hw = 12 * W2; ch = 32; break;
+    case NISQA_STAGE_CONV3: plane_layer = 4; hw = 12 * W2; ch = 64; break;
+    case NISQA_STAGE_POOL3: plane_layer = 5; hw = 6 * W3; ch = 64; break;
+    case NISQA_STAGE_CONV5: plane_layer = 6; hw = 6 * W3; ch = 64; break;
     case NISQA_STAGE_CNN_FEAT:
       if (std_mode) { src = LN.feats20.as<float>(); count = ns * 20; }
       else { src = LN.feats.as<float>(); hw = 6; ch = 64; }     // [h][c] -> c*6+h
@@ -1505,19 +1469,8 @@ int64_t nisqa_stage_dump(nisqa_engine* e, int stage, float* out, int64_t cap) {
   }
   if (ch > 0) count = ns * hw * ch;
   if (!out) return count;
-  int plane_layer = 0;          // stage lives in the plane pair feeding this conv layer
-  if (e->last_split) {
-    if (stage == NISQA_STAGE_POOL1 && e->last_conv12)
-      return fail(e, NISQA_ERR_STATE, "pool1 lives only in shared memory on the fused conv1+conv2 path: nisqa_set_option(\"conv12\", 0) before the predict call");
-    switch (stage) {
-      case NISQA_STAGE_POOL1: plane_layer = 2; break;
-      case NISQA_STAGE_POOL2: plane_layer = 3; break;
-      case NISQA_STAGE_CONV3: plane_layer = 4; break;
-      case NISQA_STAGE_POOL3: plane_layer = 5; break;
-      case NISQA_STAGE_CONV5: plane_layer = 6; break;
-      default: break;
-    }
-  }
+  if (stage == NISQA_STAGE_POOL1 && !e->last_pool1)
+    return fail(e, NISQA_ERR_STATE, "pool1 was not kept (conv12_kernel holds it in shared memory only): nisqa_set_option(\"keep_pool1\", 1) before the predict call");
   if (cap < count) return fail(e, NISQA_ERR_INVALID, "stage dump buffer too small");
   if (count == 0) return 0;
   cudaStream_t st = LN.stream;
@@ -1528,11 +1481,10 @@ int64_t nisqa_stage_dump(nisqa_engine* e, int stage, float* out, int64_t cap) {
     src = e->dump.as<float>();
   } else if (ch > 0) {
     if (plane_layer) {
-      DevBuf* tmp[7] = {nullptr, nullptr, &LN.act1, &LN.act2, &LN.act3, &LN.act4, &LN.act5};
-      CK(tmp[plane_layer]->reserve((size_t)count * 4));
+      CK(e->dump_nhwc.reserve((size_t)count * 4));
       launch_unsplit(st, std_mode, plane_layer, LN.planes[plane_layer].as<char>(),
-                     LN.planes[plane_layer].as<char>() + LN.plane_bytes[plane_layer], tmp[plane_layer]->as<float>(), (int)ns);
-      src = tmp[plane_layer]->as<float>();
+                     LN.planes[plane_layer].as<char>() + LN.plane_bytes[plane_layer], e->dump_nhwc.as<float>(), (int)ns);
+      src = e->dump_nhwc.as<float>();
     }
     CK(e->dump.reserve((size_t)count * 4));
     launch_nhwc_to_nchw(st, src, e->dump.as<float>(), ns, hw, ch);
@@ -1583,14 +1535,9 @@ int nisqa_join(nisqa_engine* e) {
 
 int nisqa_set_option(nisqa_engine* e, const char* name, int value) {
   if (!e || !name) return NISQA_ERR_INVALID;
-  if (strcmp(name, "conv_tc") == 0) { e->conv_tc = (value == 1) ? 0x7c : (value & 0x7c); return 0; }
   if (strcmp(name, "fe_ppc") == 0) { e->fe_ppc = value; return 0; }
-  if (strcmp(name, "lstm_batched") == 0) { e->lstm_batched = value != 0; return 0; }
+  if (strcmp(name, "keep_pool1") == 0) { e->keep_pool1 = value != 0; return 0; }
   if (strcmp(name, "keep_td_out") == 0) { e->keep_td_out = value != 0; return 0; }
-  if (strcmp(name, "conv12") == 0) { e->conv12 = value != 0; return 0; }
-  if (strcmp(name, "conv_split") == 0) { e->conv_split = value != 0; return 0; }
-  if (strcmp(name, "conv_pipe") == 0) { e->conv_pipe = (value == 1) ? 0x78 : (value & 0x7c); return 0; }
-  if (strcmp(name, "tc_timing_layer") == 0) { e->tc_timing_layer = value; return 0; }
   return fail(e, NISQA_ERR_INVALID, std::string("unknown option ") + name);
 }
 
@@ -1719,12 +1666,6 @@ int nisqa_gather_nccl(nisqa_engine* e, void* nccl_comm, const float* local_dev, 
 }  // extern "C"
 
 #ifdef NISQA_TC_TIMING
-extern "C" __attribute__((visibility("default"))) int nisqa_debug_tc_timing(long long* host, int n) {
-  return nisqa::tc_timing_read(host, n);
-}
-extern "C" __attribute__((visibility("default"))) int nisqa_debug_sp_timing(long long* host, int n) {
-  return nisqa::sp_timing_read(host, n);
-}
 extern "C" __attribute__((visibility("default"))) int nisqa_debug_pipe_timing(long long* host, int n, int reset) {
   return nisqa::pipe_timing_read(host, n, reset);
 }

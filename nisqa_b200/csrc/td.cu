@@ -233,111 +233,19 @@ pool_simple_kernel(const float* __restrict__ x /*[n_seg][D]*/, const ClipDesc* _
 }
 
 // ---------------------------------------------------------------------------------------
-// BiLSTM(20 -> 128), one CTA per (clip, direction), 512 threads = 512 gate rows.  The four gates
-// of hidden unit j live in one lane quad (thread t: unit t>>2, gate t&3 in PyTorch order i,f,g,o),
-// so the gate exchange is four shuffles, the cell update is replicated in the quad, and a step
-// needs ONE barrier (h and x are double buffered).  W_hh row: first 64 taps in registers, last 64
-// in shared memory [k][512].
+// BiLSTM(20 -> 128) + PoolLastStepBi
 struct LstmParams {
   const float* w_ih;   // [2][512][20]
   const float* w_hh;   // [2][512][128]
   const float* b;      // [2][512]   (bias_ih + bias_hh)
   const float* w_pool; // [256]
 };
-constexpr int kLstmSmemFloats = 64 * 512 + 2 * 128 + 2 * 32 + 128;
 
-__global__ void __launch_bounds__(512, 1)
-lstm_kernel(const float* __restrict__ feats /*[n_seg][20]*/, const ClipDesc* __restrict__ clips,
-            LstmParams P, float* __restrict__ td_out /*[n_seg][256]*/, float* __restrict__ partial /*[n_clips][2]*/) {
-  extern __shared__ __align__(16) float sm[];
-  float* whs = sm;                   // [64][512]  taps 64..127, indexed by thread
-  float* hbuf = sm + 64 * 512;       // [2][128]
-  float* xbuf = hbuf + 256;          // [2][32] input of the current / next step (20 used)
-  float* red = xbuf + 64;            // [128]
-  const int clip = blockIdx.x >> 1, dir = blockIdx.x & 1;
-  const ClipDesc cd = clips[clip];
-  const int S = cd.n_seg;
-  const int t = threadIdx.x, lane = t & 31;
-  const int unit = t >> 2, gate = t & 3;
-  const int grow = gate * 128 + unit;          // row of the PyTorch gate matrices
-  if (S <= 0) { if (t == 0) partial[clip * 2 + dir] = 0.f; return; }
-
-  float wr[64], wi[20];
-  {
-    const float* wrow = P.w_hh + ((size_t)dir * 512 + grow) * 128;
-#pragma unroll
-    for (int k = 0; k < 64; ++k) wr[k] = __ldg(wrow + k);
-    for (int k = 0; k < 64; ++k) whs[k * 512 + t] = __ldg(wrow + 64 + k);
-    const float* irow = P.w_ih + ((size_t)dir * 512 + grow) * 20;
-#pragma unroll
-    for (int k = 0; k < 20; ++k) wi[k] = __ldg(irow + k);
-  }
-  const float bias = __ldg(P.b + dir * 512 + grow);
-  if (t < 256) hbuf[t] = 0.f;
-  if (t < 64) xbuf[t] = 0.f;
-  float cstate = 0.f, hlast = 0.f;
-  const float* fb = feats + (size_t)cd.seg_off * 20;
-  __syncthreads();
-  if (t < 20) xbuf[t] = __ldg(fb + (size_t)(dir ? S - 1 : 0) * 20 + t);
-  __syncthreads();
-
-  for (int step = 0; step < S; ++step) {
-    const int tt = dir ? S - 1 - step : step;
-    const float* h = hbuf + (step & 1) * 128;
-    const float* xt = xbuf + (step & 1) * 32;
-    // prefetch the next input row while this step computes
-    float xnext = 0.f;
-    if (t < 20 && step + 1 < S) xnext = __ldg(fb + (size_t)(dir ? S - 2 - step : step + 1) * 20 + t);
-    float a0 = bias, a1 = 0.f, a2 = 0.f, a3 = 0.f;
-#pragma unroll
-    for (int k = 0; k < 20; k += 4) {
-      const float4 xv = *reinterpret_cast<const float4*>(xt + k);
-      a0 = fmaf(wi[k], xv.x, a0); a1 = fmaf(wi[k+1], xv.y, a1); a2 = fmaf(wi[k+2], xv.z, a2); a3 = fmaf(wi[k+3], xv.w, a3);
-    }
-#pragma unroll
-    for (int k = 0; k < 64; k += 4) {
-      const float4 hv = *reinterpret_cast<const float4*>(h + k);
-      a0 = fmaf(wr[k], hv.x, a0); a1 = fmaf(wr[k+1], hv.y, a1); a2 = fmaf(wr[k+2], hv.z, a2); a3 = fmaf(wr[k+3], hv.w, a3);
-    }
-#pragma unroll 8
-    for (int k = 0; k < 64; k += 4) {
-      const float4 hv = *reinterpret_cast<const float4*>(h + 64 + k);
-      a0 = fmaf(whs[(k) * 512 + t], hv.x, a0); a1 = fmaf(whs[(k+1) * 512 + t], hv.y, a1);
-      a2 = fmaf(whs[(k+2) * 512 + t], hv.z, a2); a3 = fmaf(whs[(k+3) * 512 + t], hv.w, a3);
-    }
-    const float pre = (a0 + a1) + (a2 + a3);
-    // gate nonlinearity: gate 2 is the cell candidate (tanh), the others sigmoid
-    const float act = (gate == 2) ? tanhf(pre) : 1.0f / (1.0f + expf(-pre));
-    const int q0 = lane & ~3;
-    const float ig = __shfl_sync(0xffffffffu, act, q0);
-    const float fg = __shfl_sync(0xffffffffu, act, q0 + 1);
-    const float gg = __shfl_sync(0xffffffffu, act, q0 + 2);
-    const float og = __shfl_sync(0xffffffffu, act, q0 + 3);
-    cstate = fmaf(fg, cstate, ig * gg);
-    hlast = og * tanhf(cstate);
-    if (gate == 0) {
-      hbuf[((step + 1) & 1) * 128 + unit] = hlast;
-      td_out[((size_t)cd.seg_off + tt) * 256 + dir * 128 + unit] = hlast;
-    }
-    if (t < 20) xbuf[((step + 1) & 1) * 32 + t] = xnext;
-    __syncthreads();
-  }
-  // PoolLastStepBi: this direction's final hidden state . w_pool half
-  if (gate == 0) red[unit] = hlast * __ldg(P.w_pool + dir * 128 + unit);
-  __syncthreads();
-  if (t < 32) {
-    float v = red[t] + red[t + 32] + red[t + 64] + red[t + 96];
-    v = warp_sum(v);
-    if (t == 0) partial[clip * 2 + dir] = v;
-  }
-}
-
-// ---------------------------------------------------------------------------------------
-// Batched BiLSTM (round 2): one CTA advances NB clips of one direction in lock step, so that the recurrent weights
+// One CTA advances NB clips of one direction in lock step, so that the recurrent weights
 // (512 x 128 fp32 = 256 KB: half in registers, half in shared memory) are fetched once per step for NB sequences
 // instead of once per sequence - the step is FMA bound (2 x 148 x NB FMAs per thread) instead of LDS / barrier bound,
-// and 256 clips x 2 directions fit on the chip in ONE wave (the one-sequence kernel above needed 3.5 waves of
-// 987 serial steps).  256 threads: thread t owns hidden unit u = t >> 1 and the gate pair gp = t & 1 ((i, f) or
+// and 256 clips x 2 directions fit on the chip in ONE wave (one CTA per sequence needs 3.5 waves of 987 serial
+// steps).  256 threads: thread t owns hidden unit u = t >> 1 and the gate pair gp = t & 1 ((i, f) or
 // (g, o), PyTorch row order i, f, g, o), i.e. two rows of W_hh / W_ih; the pair of lanes of a unit exchanges its four
 // gate values with two shuffles per sequence and both update the (replicated) cell state.  Sequences of a group may
 // have different lengths (clips are sorted by length on the host): a finished sequence keeps its state.
@@ -519,15 +427,6 @@ void launch_pool_final(cudaStream_t st, const float* x, const float* logits, con
   if (smem > 40 * 1024) cudaFuncSetAttribute(pool_final_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
   pool_final_kernel<<<n_clips, 64 * n_heads, smem, st>>>(x, logits, clips, P, n_heads, std::max(max_seg, 1), scores);
 }
-void launch_lstm(cudaStream_t st, const float* feats20, const ClipDesc* clips, int n_clips,
-                 const LstmParams& P, float* td_out, float* partial, float pool_bias, float* scores) {
-  static unsigned long long cfg = 0;
-  const int smem = kLstmSmemFloats * 4;
-  if (first_launch_on_device(cfg)) { cudaFuncSetAttribute(lstm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem); }
-  lstm_kernel<<<2 * n_clips, 512, smem, st>>>(feats20, clips, P, td_out, partial);
-  if (scores) lastbi_final_kernel<<<(n_clips + 127) / 128, 128, 0, st>>>(partial, clips, pool_bias, scores, n_clips);
-}
-
 void launch_pool_simple(cudaStream_t st, const float* x, int D, const ClipDesc* clips, int n_clips, int mode,
                         const PoolSimpleParams& P, int n_heads, int max_seg, float* scores) {
   const int smem = (mode == 1 ? max_seg : 0) * 4 + 16;

@@ -51,17 +51,17 @@ STAGES = [("mel_db", E.STAGE_MEL_DB, MEL_TOL_DB), ("pool1", E.STAGE_POOL1, ACT_T
     ("nisqa_mos_only.tar", [(8, 2.2, 48000), (9, 1.0, 32000)]),
     ("nisqa_tts.tar", [(10, 2.0, 16000), (11, 1.3, 48000), (12, 0.9, 22050)]),
 ])
-def test_every_stage_matches_oracle(engines, ckpt, clips):
+def test_stage_dumps_match_oracle(engines, ckpt, clips):
     eng, args, sd = engines[ckpt]
     pcm = [synth.synth_speech_pcm16(s, sec, sr) for s, sec, sr in clips]
     srs = [c[2] for c in clips]
     eng.set_option("keep_td_out", 1)              # BiLSTM: per-step outputs are only stored for the dump
-    eng.set_option("conv12", 0)                   # pool1 only exists in HBM when conv1 / conv2 run as separate kernels
+    eng.set_option("keep_pool1", 1)               # pool1 is only written to HBM for the dump
     try:
         scores, nseg, status = eng.predict_pcm(pcm, srs)
     finally:
         eng.set_option("keep_td_out", 0)
-        eng.set_option("conv12", 1)
+        eng.set_option("keep_pool1", 0)
     assert np.all(status == E.CLIP_OK)
     dumps = {name: eng.stage_dump(st) for name, st, _ in STAGES}
     off = {name: 0 for name, _, _ in STAGES}
@@ -263,67 +263,54 @@ def test_config4_full_size_tts_bs256(engines):
     ("nisqa.tar", [(31, 10.0, 48000), (32, 2.3, 48000), (33, 4.0, 16000), (34, 0.1875, 8000)]),
     ("nisqa_tts.tar", [(35, 3.0, 16000), (36, 1.1, 48000)]),
 ])
-def test_conv_paths_agree(engines, ckpt, clips):
-    """The conv2..conv6 implementations behind nisqa_set_option: fp16-plane tcgen05 pipeline as persistent
-    warp-specialised CTAs (default) and as one tile per CTA (conv_split.cu), fp32-activation tcgen05 kernels
-    (conv_tc.cu) and fp32 FFMA (cnn.cu).
-    Both tcgen05 paths do the same split and issue the same MMAs in the same order, so their scores and
-    features are BIT-identical; the FFMA path agrees to fp32 rounding noise; growing / shrinking batches
-    reuse the zero-padded planes (stale rows of earlier, larger passes must not leak)."""
+def test_keep_pool1_and_plane_reuse(engines, ckpt, clips):
+    """keep_pool1 only adds a store of pool1 for the stage dump: scores and the pool2 / pool3 / CNN-feature dumps are
+    BIT-identical with it on and off.  Growing / shrinking batches reuse the zero-padded planes (stale rows of earlier,
+    larger passes must not leak)."""
     eng, args, sd = engines[ckpt]
     pcm = [synth.synth_speech_pcm16(s, sec, sr) for s, sec, sr in clips]
     srs = [c[2] for c in clips]
     out = {}
     try:
-        for name, opts in (("planes", dict(conv_tc=1, conv_split=1, conv_pipe=1, conv12=1)),
-                           ("planes_sep12", dict(conv_tc=1, conv_split=1, conv_pipe=1, conv12=0)),
-                           ("planes_1tile", dict(conv_tc=1, conv_split=1, conv_pipe=0, conv12=0)),
-                           ("tc_f32", dict(conv_tc=1, conv_split=0)), ("ffma", dict(conv_tc=0, conv_split=0))):
-            for k, v in opts.items():
-                eng.set_option(k, v)
+        for keep in (0, 1):
+            eng.set_option("keep_pool1", keep)
             sc, nseg, st = eng.predict_pcm(pcm, srs)
-            out[name] = (sc.copy(), eng.stage_dump(E.STAGE_CNN_FEAT), eng.stage_dump(E.STAGE_POOL3), eng.stage_dump(E.STAGE_POOL2))
-        eng.set_option("conv_tc", 1); eng.set_option("conv_split", 1); eng.set_option("conv_pipe", 1); eng.set_option("conv12", 1)
-        for i in range(4):                                                          # fused conv1+conv2 == separate kernels
-            np.testing.assert_array_equal(out["planes"][i], out["planes_sep12"][i])
-        np.testing.assert_array_equal(out["planes"][0], out["planes_1tile"][0])     # persistent CTAs == one tile per CTA
-        np.testing.assert_array_equal(out["planes"][1], out["planes_1tile"][1])
-        np.testing.assert_array_equal(out["planes"][2], out["planes_1tile"][2])
-        np.testing.assert_array_equal(out["planes"][0], out["tc_f32"][0])
-        np.testing.assert_array_equal(out["planes"][1], out["tc_f32"][1])
-        assert np.abs(out["planes"][2] - out["tc_f32"][2]).max() <= 1e-5      # planes dump = hi + lo (2^-22 relative)
-        assert np.abs(out["planes"][0] - out["ffma"][0]).max() <= SCORE_TOL / 4
-        assert np.abs(out["planes"][1] - out["ffma"][1]).max() <= ACT_TOL
+            out[keep] = (sc.copy(), eng.stage_dump(E.STAGE_CNN_FEAT), eng.stage_dump(E.STAGE_POOL3), eng.stage_dump(E.STAGE_POOL2))
+        eng.set_option("keep_pool1", 0)
+        for i in range(4):
+            np.testing.assert_array_equal(out[0][i], out[1][i])
         # shrink, then grow again: same rows as in the first call
         s_small, _, _ = eng.predict_pcm(pcm[1:2], srs[1:2])
-        np.testing.assert_array_equal(s_small[0], out["planes"][0][1])
+        np.testing.assert_array_equal(s_small[0], out[0][0][1])
         s_again, _, _ = eng.predict_pcm(pcm[::-1], srs[::-1])
-        np.testing.assert_array_equal(s_again[::-1], out["planes"][0])
+        np.testing.assert_array_equal(s_again[::-1], out[0][0])
     finally:
-        eng.set_option("conv_tc", 1); eng.set_option("conv_split", 1); eng.set_option("conv_pipe", 1); eng.set_option("conv12", 1)
+        eng.set_option("keep_pool1", 0)
 
 
-def test_lstm_paths_agree(engines):
-    """Batched BiLSTM (NB clips of one direction per CTA, sorted by length) against the one-sequence kernel: the same
-    fp32 dot products in a different summation order -> scores within fp32 noise; ragged lengths inside a group, a
-    too-short clip (no segments) and batch sizes that select the NB = 1, 2 and 4 variants."""
+def test_removed_kernel_switches_are_rejected(engines):
+    """Each stage has one implementation: the former A/B switches are unknown options, not silent no-ops."""
+    eng = engines["nisqa.tar"][0]
+    for name in ("conv_tc", "conv_split", "conv_pipe", "conv12", "lstm_batched", "td_tiled"):
+        with pytest.raises(E.EngineError, match="unknown option"):
+            eng.set_option(name, 1)
+
+
+def test_batched_lstm_matches_oracle(engines):
+    """Batched BiLSTM (NB clips of one direction per CTA, sorted by length) against the oracle: ragged lengths inside a
+    group, a too-short clip (no segments) and batch sizes that select the NB = 1, 2 and 4 variants."""
     eng, args, sd = engines["nisqa_tts.tar"]
     spec = [(61, 10.0, 16000), (62, 0.5, 16000), (63, 3.3, 48000), (64, 0.01, 16000), (65, 6.1, 22050), (66, 2.0, 16000), (67, 1.1, 8000)]
     base = [synth.synth_speech_pcm16(s, sec, sr) for s, sec, sr in spec]
+    ref = [O.predict_pcm(args, sd, _f32(p), sr)[0] for p, (_, _, sr) in zip(base, spec)]     # once per distinct clip
     for reps in (1, 25, 50):                      # 7, 175, 350 clips -> 14, 350, 700 sequences: NB = 1, 4 (> 296) / 2
         pcm = base * reps
         srs = [c[2] for c in spec] * reps
-        try:
-            eng.set_option("lstm_batched", 0)
-            s0, n0, st0 = eng.predict_pcm(pcm, srs)
-            eng.set_option("lstm_batched", 1)
-            s1, n1, st1 = eng.predict_pcm(pcm, srs)
-        finally:
-            eng.set_option("lstm_batched", 1)
-        np.testing.assert_array_equal(st0, st1)
-        np.testing.assert_array_equal(np.isnan(s0), np.isnan(s1))
+        s1, n1, st1 = eng.predict_pcm(pcm, srs)
         ok = st1 == E.CLIP_OK
-        assert np.abs(s0[ok] - s1[ok]).max() <= 2e-5, float(np.abs(s0[ok] - s1[ok]).max())
+        assert np.all(np.isnan(s1[~ok]))
+        for i in np.nonzero(ok)[0]:
+            assert np.abs(s1[i] - ref[i % 7]).max() <= SCORE_TOL, (reps, int(i), float(np.abs(s1[i] - ref[i % 7]).max()))
         assert st1[3] == E.CLIP_TOO_SHORT and np.isnan(s1[3, 0])
         np.testing.assert_array_equal(s1[:7], s1[7 * (reps - 1):])     # the same clip scores the same in any group
     pcm = base[:5] * 30                              # 150 clips -> 300 sequences: NB = 4

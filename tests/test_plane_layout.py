@@ -187,7 +187,7 @@ def test_implicit_gemm_over_shifted_tiles_is_conv2d(name, H, W, C, pool, pow_, c
         # conv_split.cu order: positions x channels
         D = implicit_gemm(X, w_sum, g)
         tol = 2e-5          # weights enter as w_hi + w_lo (2^-22 of |w|), accumulation in float64 here
-        # conv_split.cu's epilogue: thread <-> tile row r = s*BLK + hh*P + ww (interior rows only)
+        # conv_pipe_kernel's epilogue: thread <-> tile row r = s*BLK + hh*P + ww (interior rows only)
         for s in range(live):
             for h in range(H):
                 for w in range(W):
@@ -198,7 +198,7 @@ def test_implicit_gemm_over_shifted_tiles_is_conv2d(name, H, W, C, pool, pow_, c
                     if not pool:
                         np.testing.assert_allclose(v, ref[seg0 + s, h, 0 if center else w], rtol=0, atol=tol)
             if pool:
-                # epilogue part 2 of conv_split.cu: max over the staged interior rows of each pooling window
+                # pooling epilogue of conv_pipe_kernel: max over the staged interior rows of each pooling window
                 # (adaptive windows [floor(pw*W/POW), ceil((pw+1)*W/POW)) or 2x2)
                 for ph in range(H // 2):
                     for pw in range(pow_):

@@ -25,23 +25,14 @@ STALL_NAMES = ["long_scoreboard", "short_scoreboard", "barrier", "math_pipe_thro
 
 
 def short(name, seen):
-    table = [("conv12", "conv12"), ("frontend", "frontend"), ("seg_table", "seg_table"), ("conv1_pool1", "conv1"),
+    table = [("conv12", "conv12"), ("frontend", "frontend"), ("seg_table", "seg_table"), ("conv1_pool1", "pool1_dump"),
              ("linear_rows_kernel<64", "lin_ln"), ("linear_rows_kernel<20", "fc_out"), ("qkv", "qkv"),
              ("sa_layer", "sa_layer"), ("pool_logits", "pool_logits"), ("pool_final", "pool_final"),
              ("lstm", "lstm"), ("lastbi", "lastbi")]
     name = name.replace("(int)", "").replace("(bool)", "")
-    m = re.search(r"SpCfg<(\d+), (\d+), (\d+), (\d+), (\d+), (\d+), (\d+), (\d+), (\w+), (\w+)>", name)
+    m = re.search(r"conv_pipe_kernel<nisqa::SpCfg<[^>]*>, (\d+)>", name)
     if m:
-        h, ci, f32out = int(m.group(1)), int(m.group(3)), m.group(9) in ("1", "true")
-        layer = {(24, 16): 2, (12, 32): 3, (12, 64): 4}.get((h, ci))
-        return "conv%d" % (layer if layer else (6 if f32out else 5))
-    m = re.search(r"TcCfg<(\d+), (\d+), (\d+), (\d+), (\d+), (\d+), (\d+), (\d+)", name)
-    if m:
-        h, w, ci, co, pool, pw, ns, center = [int(x) for x in m.groups()]
-        layer = {(24, 16): 2, (12, 32): 3, (12, 64): 4}.get((h, ci))
-        if layer is None:
-            layer = 6 if (center or "conv5" in seen) else 5
-        return "conv%d" % layer
+        return "conv%s" % m.group(1)
     for k, v in table:
         if k in name:
             return v

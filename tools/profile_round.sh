@@ -8,23 +8,6 @@ OUT=gpurun_out
 mkdir -p $OUT
 BENCH_PROF="python bench.py --steps 2 --warmup 1 --warmup-seconds 0 --skip-cpu"
 python -c "import torch" 2>/dev/null     # page the image in
-# optional A/B of prebuilt variants (nisqa_b200/exp/libnisqa_<name>.so, tools/tc_ab_build.sh) against the
-# default build: the faster library is the one everything below runs with; the choice is logged so that
-# the source default can follow it
-if [ -n "$AB_VARIANT" ] && [ -f nisqa_b200/exp/libnisqa_$AB_VARIANT.so ]; then
-  timeout 150 python tools/tc_ab.py --split 1 --skip-check --tag default > $OUT/${TAG}_ab.log 2>&1
-  timeout 150 python tools/tc_ab.py --split 1 --skip-check --lib nisqa_b200/exp/libnisqa_$AB_VARIANT.so --tag $AB_VARIANT >> $OUT/${TAG}_ab.log 2>&1
-  timeout 150 python tools/tc_ab.py --split 1 --skip-check --timing --lib nisqa_b200/exp/libnisqa_timing.so --tag T_default >> $OUT/${TAG}_ab.log 2>&1
-  grep -v Warning $OUT/${TAG}_ab.log | grep "clips/s\|conv"
-  D=$(grep "^\[default\]" $OUT/${TAG}_ab.log | sed 's/.*\] \([0-9]*\) clips.*/\1/')
-  V=$(grep "^\[$AB_VARIANT\]" $OUT/${TAG}_ab.log | sed 's/.*\] \([0-9]*\) clips.*/\1/')
-  if [ -n "$D" ] && [ -n "$V" ] && [ "$V" -gt $((D + D / 100)) ]; then
-    cp nisqa_b200/exp/libnisqa_$AB_VARIANT.so nisqa_b200/libnisqa_b200.so
-    echo "AB_CHOICE=$AB_VARIANT ($V vs default $D clips/s)" | tee $OUT/${TAG}_ab_choice.txt
-  else
-    echo "AB_CHOICE=default ($D vs $AB_VARIANT $V clips/s)" | tee $OUT/${TAG}_ab_choice.txt
-  fi
-fi
 timeout 600 python -m pytest tests -m gpu -x -q > $OUT/${TAG}_pytest.log 2>&1
 echo "pytest exit $?"; tail -3 $OUT/${TAG}_pytest.log
 # full capture of one step (LPS launches per step; the first step is skipped), raw page exported on the box; the

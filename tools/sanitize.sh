@@ -1,7 +1,7 @@
 #!/bin/bash
 # GPU-box memory / race / init check of every kernel on the default path (SURVEY.md section 5: the reference has no
 # sanitizer story; this is ours): compute-sanitizer memcheck over __graft_entry__.smoke() (nisqa.tar, two
-# short clips at 48 / 16 kHz: front-end, conv1, the five tcgen05 conv layers with their bulk copies /
+# short clips at 48 / 16 kHz: front-end, conv1 + conv2 fused, the tcgen05 conv3..conv6 with their bulk copies /
 # mbarriers / TMEM, self-attention, pooling) and over a short nisqa_tts.tar call (StandardCNN, BiLSTM).
 #   gpurun --timeout 300 -- 'bash tools/sanitize.sh r01e'
 TAG=${1:-rXX}

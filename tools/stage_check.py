@@ -20,6 +20,7 @@ def check(ckpt, clips):
     std = args["cnn_model"] == "standard"
     pcm = [synth.synth_speech_pcm16(s, sec, sr) for (s, sec, sr) in clips]
     srs = [c[2] for c in clips]
+    eng.set_option("keep_pool1", 1)       # pool1 is only written to HBM for the dump
     t0 = time.time()
     scores, nseg, status = eng.predict_pcm(pcm, srs)
     print("== %s: predict %.3fs  status=%s nseg=%s launches=%d" % (ckpt, time.time() - t0, status.tolist(), nseg.tolist(), eng.kernel_launches()))

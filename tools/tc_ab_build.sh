@@ -3,7 +3,7 @@
 set -e
 cd "$(dirname "$0")/.."
 F="-gencode arch=compute_100a,code=sm_100a -O3 -std=c++17 -lineinfo -Xcompiler -fPIC -Xcompiler -fvisibility=hidden --shared"
-S="nisqa_b200/csrc/engine.cu nisqa_b200/csrc/frontend.cu nisqa_b200/csrc/cnn.cu nisqa_b200/csrc/conv_tc.cu nisqa_b200/csrc/conv_split.cu nisqa_b200/csrc/conv12.cu nisqa_b200/csrc/td.cu nisqa_b200/csrc/td_tiled.cu nisqa_b200/csrc/wavio.cpp nisqa_b200/csrc/flac.cpp nisqa_b200/csrc/resample.cpp nisqa_b200/csrc/resample_gpu.cu"
+S=$(python -c "from nisqa_b200 import build as b; print(' '.join('nisqa_b200/csrc/' + f for f in b.SOURCES))")
 mkdir -p nisqa_b200/exp
 nvcc $F -DNISQA_TC_TIMING $S -o nisqa_b200/exp/libnisqa_timing.so -ldl &
 for v in "$@"; do     # extra variants: name=-DFLAG[,-DFLAG2]
