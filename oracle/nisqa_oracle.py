@@ -7,6 +7,11 @@ as the CPU baseline being timed.  The product path (``nisqa_b200/``) never impor
 What it is: a per-clip, unpadded restatement of the reference's predict path in NumPy +
 torch-CPU functional ops (the same arithmetic library the reference uses on the CPU), each
 function citing the reference ``file:line`` it follows (``lib`` = nisqa/NISQA_lib.py).
+The model half follows the dtype of its inputs: float32 by default (the reference's own
+arithmetic), float64 with ``state_dict_as(sd, torch.float64)`` and float64 inputs.  Its
+per-layer entry points (``conv_layer``, ``cnn_head``, ``sa_input``, ``sa_layer``, ``bilstm``,
+``pool_heads``) are what the whole-model functions are built from, so a single kernel can be
+held to a restatement of exactly its own layer (tests/test_kernel_precision.py).
 
 Pinning status
   * model half (segments -> scores): PINNED against the unmodified reference modules imported
@@ -35,6 +40,12 @@ def load_checkpoint(path):
     ck = torch.load(path, map_location="cpu", weights_only=False)
     sd = {k: v.detach().clone() for k, v in ck["model_state_dict"].items()}
     return dict(ck["args"]), sd
+
+
+def state_dict_as(sd, dtype):
+    """The floating-point tensors of a state_dict cast to ``dtype`` (unfolded, as stored in the checkpoint): the model
+    half is dtype-generic, so ``state_dict_as(sd, torch.float64)`` with float64 inputs restates it in float64."""
+    return {k: (v.to(dtype) if v.is_floating_point() else v) for k, v in sd.items()}
 
 
 # ------------------------------------------------------------------ front-end (a1-a6)
@@ -69,10 +80,10 @@ def segment_counts(n_samples, sr, args):
     return n_frames, n_seg, STATUS_OK
 
 
-def segments(spec, args):
+def segments(spec, args, dtype=torch.float32):
     """lib:2239-2273 without the zero-padding tail: x[i,0,m,t] = spec[m, i*seg_hop + t]."""
     seg_len, seg_hop = args["ms_seg_length"], args["ms_seg_hop_length"]
-    spec = torch.as_tensor(np.ascontiguousarray(spec), dtype=torch.float32)
+    spec = torch.as_tensor(np.ascontiguousarray(spec), dtype=dtype)
     n_wins = spec.shape[1] - (seg_len - 1)
     if n_wins < 1:
         raise ValueError("Sample too short")
@@ -92,48 +103,52 @@ def _conv_bn_relu(sd, i, x, padding):
     return F.relu(x)
 
 
-def adapt_cnn(sd, x, args, taps=None):
-    """lib:688-710 (eval mode: Dropout2d is the identity)."""
-    x = _conv_bn_relu(sd, 1, x, (1, 1))
-    x = F.adaptive_max_pool2d(x, output_size=tuple(args["cnn_pool_1"]))
-    if taps is not None: taps["pool1"] = x
-    x = _conv_bn_relu(sd, 2, x, (1, 1))
-    x = F.adaptive_max_pool2d(x, output_size=tuple(args["cnn_pool_2"]))
-    if taps is not None: taps["pool2"] = x
-    x = _conv_bn_relu(sd, 3, x, (1, 1))
-    if taps is not None: taps["conv3"] = x
-    x = _conv_bn_relu(sd, 4, x, (1, 1))
-    x = F.adaptive_max_pool2d(x, output_size=tuple(args["cnn_pool_3"]))
-    if taps is not None: taps["pool3"] = x
-    x = _conv_bn_relu(sd, 5, x, (1, 1))
-    if taps is not None: taps["conv5"] = x
-    x = _conv_bn_relu(sd, 6, x, (1, 0))          # kernel (3, pool_3[1]) pad (1,0): W 3 -> 1
-    x = x.reshape(-1, 64 * args["cnn_pool_3"][0])
-    if "cnn.model.fc.weight" in sd:              # cnn_fc_out_h (lib:682-684, 708-709)
-        x = F.linear(x, sd["cnn.model.fc.weight"], sd["cnn.model.fc.bias"])
-    return x
+def conv_layer(sd, i, x, args):
+    """conv i + BN + ReLU, followed by the max-pool that belongs to that layer (pool1 / pool2 / pool3 behind conv 1 / 2
+    / 4), of the AdaptCNN (lib:688-706, eval mode: Dropout2d is the identity) or the StandardCNN (lib:811-830: fixed
+    MaxPool2d(2), the first one with padding (0,1))."""
+    return cnn_pool(i, _conv_bn_relu(sd, i, x, conv_padding(i, args)), args)
 
 
-def standard_cnn(sd, x, args, taps=None):
-    """lib:811-836: fixed MaxPool2d(2) (first with padding (0,1)), fc_out 768 -> 20."""
-    x = _conv_bn_relu(sd, 1, x, 1)
-    x = F.max_pool2d(x, 2, stride=2, padding=(0, 1))
-    if taps is not None: taps["pool1"] = x
-    x = _conv_bn_relu(sd, 2, x, 1)
-    x = F.max_pool2d(x, 2, stride=2)
-    if taps is not None: taps["pool2"] = x
-    x = _conv_bn_relu(sd, 3, x, 1)
-    if taps is not None: taps["conv3"] = x
-    x = _conv_bn_relu(sd, 4, x, 1)
-    x = F.max_pool2d(x, 2, stride=2)
-    if taps is not None: taps["pool3"] = x
-    x = _conv_bn_relu(sd, 5, x, 1)
-    if taps is not None: taps["conv5"] = x
-    x = _conv_bn_relu(sd, 6, x, 1)
+def conv_padding(i, args):
+    if args["cnn_model"] == "adapt" and i == 6:
+        return (1, 0)                            # conv6: kernel (3, pool_3[1]) pad (1,0): W 3 -> 1
+    return (1, 1)
+
+
+def cnn_pool(i, x, args):
+    """The max-pool behind conv i (the identity behind conv 3, 5 and 6)."""
+    if args["cnn_model"] == "adapt":
+        pool = {1: "cnn_pool_1", 2: "cnn_pool_2", 4: "cnn_pool_3"}.get(i)
+        return F.adaptive_max_pool2d(x, output_size=tuple(args[pool])) if pool else x
+    if i == 1:
+        return F.max_pool2d(x, 2, stride=2, padding=(0, 1))
+    return F.max_pool2d(x, 2, stride=2) if i in (2, 4) else x
+
+
+def cnn_head(sd, x, args):
+    """conv6's output -> the framewise features: flatten (lib:707, 831) and the optional Linear (AdaptCNN cnn_fc_out_h,
+    lib:708-709; StandardCNN fc_out 768 -> 20, lib:832-834)."""
+    if args["cnn_model"] == "adapt":
+        x = x.reshape(-1, 64 * args["cnn_pool_3"][0])
+        if "cnn.model.fc.weight" in sd:
+            x = F.linear(x, sd["cnn.model.fc.weight"], sd["cnn.model.fc.bias"])
+        return x
     x = x.reshape(-1, 64 * 6 * 2)
     if "cnn.model.fc_out.weight" in sd:
         x = F.linear(x, sd["cnn.model.fc_out.weight"], sd["cnn.model.fc_out.bias"])
     return x
+
+
+_CNN_TAPS = {1: "pool1", 2: "pool2", 3: "conv3", 4: "pool3", 5: "conv5"}
+
+
+def conv_cnn(sd, x, args, taps=None):
+    """AdaptCNN (lib:688-710) or StandardCNN (lib:811-836): six conv_layer()s and cnn_head()."""
+    for i in range(1, 7):
+        x = conv_layer(sd, i, x, args)
+        if taps is not None and i in _CNN_TAPS: taps[_CNN_TAPS[i]] = x
+    return cnn_head(sd, x, args)
 
 
 def skip_cnn(sd, x):
@@ -164,27 +179,42 @@ def self_attention(sd, feats, taps=None, pos_enc=False):
 
     nn.MultiheadAttention with one head: q,k,v = in_proj; q *= 1/sqrt(64); softmax(q k^T) v;
     out_proj; post-norm residual blocks."""
+    x = sa_input(sd, feats, pos_enc, taps)
+    for l in range(sa_layers(sd)):
+        x = sa_layer(sd, l, x)
+        if taps is not None: taps["sa_l%d" % l] = x
+    return x
+
+
+def sa_input(sd, feats, pos_enc=False, taps=None):
+    """The input block of SelfAttention (lib:1025-1029) for ONE clip: Linear, LayerNorm, then the positional encoding
+    (lib:1042-1062: x + pe[:S] with the registered buffer [max_len, 1, d]; eval: no dropout)."""
     p = "time_dependency.model."
     x = F.linear(feats, sd[p + "linear.weight"], sd[p + "linear.bias"])
     x = F.layer_norm(x, (x.shape[-1],), sd[p + "norm1.weight"], sd[p + "norm1.bias"], 1e-5)
     if taps is not None: taps["sa_in"] = x
     if pos_enc:
-        # PositionalEncoding (lib:1042-1062): x + pe[:S] with the registered buffer [max_len, 1, d] (eval: no dropout)
         x = x + sd[p + "pos_encoder.pe"][:x.shape[0], 0, :]
-    n_layers = len({k.split(".")[3] for k in sd if k.startswith(p + "layers.")})
-    for l in range(n_layers):
-        q = p + "layers.%d." % l
-        d = x.shape[-1]
-        qkv = F.linear(x, sd[q + "self_attn.in_proj_weight"], sd[q + "self_attn.in_proj_bias"])
-        qq, kk, vv = qkv[:, :d], qkv[:, d:2 * d], qkv[:, 2 * d:]
-        att = torch.softmax((qq * (1.0 / math.sqrt(d))) @ kk.t(), dim=-1)
-        sa = F.linear(att @ vv, sd[q + "self_attn.out_proj.weight"], sd[q + "self_attn.out_proj.bias"])
-        x = F.layer_norm(x + sa, (d,), sd[q + "norm1.weight"], sd[q + "norm1.bias"], 1e-5)
-        ff = F.linear(F.relu(F.linear(x, sd[q + "linear1.weight"], sd[q + "linear1.bias"])),
-                      sd[q + "linear2.weight"], sd[q + "linear2.bias"])
-        x = F.layer_norm(x + ff, (d,), sd[q + "norm2.weight"], sd[q + "norm2.bias"], 1e-5)
-        if taps is not None: taps["sa_l%d" % l] = x
     return x
+
+
+def sa_layers(sd):
+    p = "time_dependency.model.layers."
+    return len({k.split(".")[3] for k in sd if k.startswith(p)})
+
+
+def sa_layer(sd, l, x):
+    """Encoder layer l of SelfAttention (lib:988-996, 1030-1040) for ONE clip."""
+    q = "time_dependency.model.layers.%d." % l
+    d = x.shape[-1]
+    qkv = F.linear(x, sd[q + "self_attn.in_proj_weight"], sd[q + "self_attn.in_proj_bias"])
+    qq, kk, vv = qkv[:, :d], qkv[:, d:2 * d], qkv[:, 2 * d:]
+    att = torch.softmax((qq * (1.0 / math.sqrt(d))) @ kk.t(), dim=-1)
+    sa = F.linear(att @ vv, sd[q + "self_attn.out_proj.weight"], sd[q + "self_attn.out_proj.bias"])
+    x = F.layer_norm(x + sa, (d,), sd[q + "norm1.weight"], sd[q + "norm1.bias"], 1e-5)
+    ff = F.linear(F.relu(F.linear(x, sd[q + "linear1.weight"], sd[q + "linear1.bias"])),
+                  sd[q + "linear2.weight"], sd[q + "linear2.bias"])
+    return F.layer_norm(x + ff, (d,), sd[q + "norm2.weight"], sd[q + "norm2.bias"], 1e-5)
 
 
 def bilstm(sd, feats):
@@ -198,9 +228,9 @@ def bilstm(sd, feats):
         b = sd[p + "bias_ih_l0" + suffix] + sd[p + "bias_hh_l0" + suffix]
         H = w_hh.shape[1]
         gx = feats @ w_ih.t() + b
-        h = torch.zeros(H)
-        c = torch.zeros(H)
-        out = torch.zeros(S, H)
+        h = torch.zeros(H, dtype=feats.dtype)
+        c = torch.zeros(H, dtype=feats.dtype)
+        out = torch.zeros(S, H, dtype=feats.dtype)
         for t in order:
             g = gx[t] + w_hh @ h
             i, f, gg, o = g[:H], g[H:2 * H], g[2 * H:3 * H], g[3 * H:]
@@ -262,7 +292,7 @@ def forward_de_from_mel(args, sd, spec, spec_ref, taps=None):
     with torch.no_grad():
         outs = []
         for sp in (spec, spec_ref):
-            feats = adapt_cnn(sd, segments(sp, args), args)
+            feats = conv_cnn(sd, segments(sp, args), args)
             outs.append(self_attention(sd, feats, pos_enc=bool(args.get("td_sa_pos_enc"))))
         x, y = outs
         y_al = de_align(args, x, y, sd)
@@ -340,10 +370,8 @@ def forward_from_mel(args, sd, spec, taps=None):
     x = segments(spec, args)
     if taps is not None: taps["n_segments"] = x.shape[0]
     with torch.no_grad():
-        if args["cnn_model"] == "adapt":
-            feats = adapt_cnn(sd, x, args, taps)
-        elif args["cnn_model"] == "standard":
-            feats = standard_cnn(sd, x, args, taps)
+        if args["cnn_model"] in ("adapt", "standard"):
+            feats = conv_cnn(sd, x, args, taps)
         elif args["cnn_model"] in (None, "skip"):
             feats = skip_cnn(sd, x)
         elif args["cnn_model"] == "dff":
@@ -364,21 +392,27 @@ def forward_from_mel(args, sd, spec, taps=None):
         elif args.get("td_2") not in (None, "skip"):
             raise NotImplementedError(args["td_2"])
         if taps is not None: taps["td_out"] = td
-        if args["model"] == "NISQA_DIM":
-            prefixes = ["pool_layers.%d.model." % i for i in range(5)]
+        return pool_heads(args, sd, td).numpy()
+
+
+def pool_heads(args, sd, td):
+    """The pooling module(s) of ONE clip (lib:255-266): five heads for NISQA_DIM (order mos,noi,dis,col,loud), one
+    otherwise -> scores [5] or [1]."""
+    if args["model"] == "NISQA_DIM":
+        prefixes = ["pool_layers.%d.model." % i for i in range(5)]
+    else:
+        prefixes = ["pool.model."]
+    outs = []
+    for pf in prefixes:
+        if args["pool"] == "att":
+            outs.append(pool_attff(sd, pf, td) if args.get("pool_att_h") else pool_att(sd, pf, td))
+        elif args["pool"] == "last_step_bi":
+            outs.append(pool_last_step_bi(sd, pf, td))
+        elif args["pool"] in ("avg", "max", "last_step"):
+            outs.append({"avg": pool_avg, "max": pool_max, "last_step": pool_last_step}[args["pool"]](sd, pf, td))
         else:
-            prefixes = ["pool.model."]
-        outs = []
-        for pf in prefixes:
-            if args["pool"] == "att":
-                outs.append(pool_attff(sd, pf, td) if args.get("pool_att_h") else pool_att(sd, pf, td))
-            elif args["pool"] == "last_step_bi":
-                outs.append(pool_last_step_bi(sd, pf, td))
-            elif args["pool"] in ("avg", "max", "last_step"):
-                outs.append({"avg": pool_avg, "max": pool_max, "last_step": pool_last_step}[args["pool"]](sd, pf, td))
-            else:
-                raise NotImplementedError(args["pool"])
-    return torch.cat(outs).numpy()
+            raise NotImplementedError(args["pool"])
+    return torch.cat(outs)
 
 
 def predict_pcm(args, sd, y, sr, taps=None):
